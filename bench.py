@@ -2,7 +2,7 @@
 """bench.py — DuoDiff sampling throughput (images/sec, 1000 DDPM steps, t_switch=300) on N B200s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config celeba] [--batch 128]
-                    [--ee [--threshold 0.08] [--slope 0.5]] [--decode] [--verify-shards]
+                    [--ee [--threshold 0.08] [--slope 0.5]] [--decode] [--verify-shards] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: a full 1000-step DuoDiff sampling of `batch` images per GPU
 (300 shallow-U-ViT steps, 700 full-U-ViT steps, 1000 DDPM updates).  One JSON line on stdout (rank 0):
@@ -17,6 +17,8 @@ A "step" is one pass of the hot path over one batch: a full 1000-step DuoDiff sa
 `--impl reference` times the reference's own CPU implementation of the path instead (see DESIGN.md §5).
 `--ee` measures BASELINE config 3 (DeeDiff early exit, compaction mode) instead of the DuoDiff pair.
 `--verify-shards` is a correctness run, not a benchmark: N-rank sharded sampling == single-GPU sampling row for row.
+`--dump-outputs DIR` writes what the timed path returned in its last timed step as DIR/<name>.npy (see dump_outputs):
+the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -109,6 +111,29 @@ def workload_config(name: str, B: int, world: int, extra: str = "") -> dict:
                 l2="no flush: one DDPM step touches ~1 GB of activations+weights (> 126 MB L2)")
 
 
+DUMP_LIMIT = 64 << 20  # bytes of .npy data per --dump-outputs directory
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write each array as out_dir/<name>.npy in float32 (integer logs converted), at most DUMP_LIMIT bytes in all.
+    Smaller arrays are written whole; one that does not fit its share of what is left is replaced by a fixed sample of
+    its rows (leading dimension, seed 0, kept in order), so that the same arguments always select the same rows."""
+    import numpy as np
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    items = sorted(((k, v.detach().float().cpu().numpy()) for k, v in arrays.items()), key=lambda kv: kv[1].nbytes)
+    left = DUMP_LIMIT
+    for i, (name, a) in enumerate(items):
+        share = left // (len(items) - i) - 4096  # headroom for the .npy header
+        if a.nbytes > share:
+            keep = share // a[0].nbytes
+            if keep < 1:
+                raise ValueError(f"--dump-outputs: one row of {name} {a.shape} exceeds {share} bytes")
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(d / f"{name}.npy", a)
+        left -= (d / f"{name}.npy").stat().st_size
+
+
 class ClockSampler:
     """nvidia-smi clocks + throttle reasons sampled every 200 ms while the timed region runs."""
     Q = ("clocks.sm,clocks.max.sm,clocks_event_reasons.hw_slowdown,clocks_event_reasons.hw_thermal_slowdown,"
@@ -195,7 +220,7 @@ def run_reference(args, rank: int, world: int) -> None:
     sampler.get_samples for all 1000 steps instead (BASELINE config 1: CIFAR-10, batch 8)."""
     if rank != 0:
         return
-    steps, warm = max(args.steps, 1), max(args.warmup, 0)
+    steps, warm = args.steps, args.warmup
     torch.set_num_threads(max(1, os.cpu_count() or 1))  # torchrun exports OMP_NUM_THREADS=1
     shallow, full, default_b = PAIRS[args.config]
     B = args.batch or default_b
@@ -402,6 +427,8 @@ def run_ours(args, rank: int, world: int, local_rank: int) -> None:
     launches = lib.ddb_launch_count() - l0
     ms = e0.elapsed_time(e1)
     assert torch.isfinite(out).all(), "non-finite samples"
+    if args.dump_outputs and rank == 0:  # the finished samples of the whole job, [world*B, H, W, C] (NHWC, in [0, 1])
+        dump_outputs(args.dump_outputs, dict(samples=torch.cat(gathered) if world > 1 else out))
 
     # ---- end-to-end through the public API (host x_T -> H2D -> 1000 steps -> NHWC -> D2H numpy)
     def e2e_pass(i: int):
@@ -583,6 +610,8 @@ def run_ee(args, rank: int, world: int, local_rank: int) -> None:
     launches = lib.ddb_launch_count() - l0
     ms = e0.elapsed_time(e1)
     assert torch.isfinite(out).all()
+    if args.dump_outputs and rank == 0:  # rank 0's shard; the side measurements below overwrite both logs
+        dump_outputs(args.dump_outputs, dict(samples=out, exit_log=exit_log, score_log=score_log))
     idx = exit_log.float()  # [1000, B] of the last pass
     mean_exit = idx.mean().item()
     exit_hist = torch.bincount(exit_log.flatten().long().cpu(), minlength=depth + 1).tolist()
@@ -758,7 +787,13 @@ def main():
     ap.add_argument("--full-run", action="store_true",
                     help="--impl reference: run the unmodified get_samples for all 1000 steps (config 1: --config cifar10 --batch 8)")
     ap.add_argument("--verify-shards", action="store_true", help="N-rank sharded == single-GPU, row for row (not a benchmark)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, <= 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl == "reference" or args.verify_shards):
+        ap.error("--dump-outputs records the GPU sampling path: not with --impl reference or --verify-shards")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))

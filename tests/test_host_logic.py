@@ -275,6 +275,34 @@ def test_bench_reference_arm_contract():
     assert d["value"] > 0 and d["gpu_launches"] == 0
 
 
+def test_bench_dump_outputs_fit_the_limit_and_repeat(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: float32 .npy files within DUMP_LIMIT bytes in all; an array that fits is written
+    whole, a larger one as the same seeded sample of its rows on every call."""
+    import importlib.util
+    import subprocess
+    import sys
+    spec = importlib.util.spec_from_file_location("_bench", ROOT / "bench.py")
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    monkeypatch.setattr(bench, "DUMP_LIMIT", 1 << 20)
+    g = torch.Generator().manual_seed(0)
+    samples = torch.rand(80, 32, 32, 3, generator=g)  # 960 KB
+    exit_log = torch.randint(0, 13, (1000, 80), generator=g, dtype=torch.int32)  # 312 KB
+    bench.dump_outputs(str(tmp_path), dict(samples=samples, exit_log=exit_log))
+    files = sorted(tmp_path.iterdir())
+    assert [p.name for p in files] == ["exit_log.npy", "samples.npy"]
+    assert sum(p.stat().st_size for p in files) <= 1 << 20
+    log, got = np.load(tmp_path / "exit_log.npy"), np.load(tmp_path / "samples.npy")
+    assert log.dtype == got.dtype == np.float32 and np.array_equal(log, exit_log.numpy())
+    assert 0 < len(got) < 80 and got.shape[1:] == (32, 32, 3)
+    rows = [i for r in got for i in range(80) if np.array_equal(r, samples[i].numpy())]
+    assert rows == sorted(set(rows)) and len(rows) == len(got)  # distinct rows of the output, in order
+    bench.dump_outputs(str(tmp_path), dict(samples=samples, exit_log=exit_log))
+    assert np.array_equal(np.load(tmp_path / "samples.npy"), got)
+    res = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--steps", "0"], capture_output=True, text=True)
+    assert res.returncode == 2 and "--steps" in res.stderr
+
+
 def test_cli_labels_follow_the_reference_draw_modulo_num_classes():
     """sampler.py:314-318: `--class_id` draws torch.randint(1, 1001, (B,)) after seed_everything(seed).  The shims keep
     that draw and take it modulo num_classes (documented deviation: label 1000 cannot index a 1000-row table)."""
