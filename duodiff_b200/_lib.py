@@ -67,6 +67,13 @@ _SIGS = {
     "ddb_ae_num_ops": (C.c_int32, [_P]),
     "ddb_ae_op_info": (C.c_int, [_P, C.c_int32, C.c_char_p, C.c_int32, _P]),
     "ddb_ae_decode_debug": (C.c_int, [_P, _P, C.c_int32, _P, C.c_int32, _P, _P]),
+    "ddb_ae_create_encoder": (C.c_int, [_P, C.POINTER(Tensor), C.c_int32]),
+    "ddb_ae_encode_moments": (C.c_int, [_P, _P, C.c_int32, _P, _P]),
+    "ddb_ae_sample": (C.c_int, [_P, _P, _P, C.c_int32, _P, _P]),
+    "ddb_ae_profile_encode": (C.c_int, [_P, _P, C.c_int32, _P, _P, _P, _P]),
+    "ddb_ae_encoder_num_ops": (C.c_int32, [_P]),
+    "ddb_ae_encoder_op_info": (C.c_int, [_P, C.c_int32, C.c_char_p, C.c_int32, _P]),
+    "ddb_ae_encode_debug": (C.c_int, [_P, _P, C.c_int32, _P, C.c_int32, _P, _P]),
     "ddb_op_pack_linear": (C.c_int, [_P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGS)

@@ -1,10 +1,11 @@
-"""Drop-in for the decode side of the reference's ``models/utils/autoencoder.py`` (``FrozenAutoencoderKL`` :452-500,
-``get_autoencoder`` :503-516): the latent -> image decoder that ``sampler.get_samples`` / ``eesampler.get_samples``
-call after the last denoising step of a latent model (sampler.py:141-143, eesampler.py:84-85).
+"""Drop-in for the reference's ``models/utils/autoencoder.py`` (``FrozenAutoencoderKL`` :452-500, ``get_autoencoder``
+:503-516): the latent -> image decoder that ``sampler.get_samples`` / ``eesampler.get_samples`` call after the last
+denoising step of a latent model (sampler.py:141-143, eesampler.py:84-85), and the image -> latent encoder
+(``encode_moments`` / ``sample`` / ``encode``) used to prepare latents and to check reconstructions.
 
 All arithmetic runs inside libduodiff_b200.so (implicit-GEMM tcgen05 convolutions, csrc/conv_gemm.cuh); PyTorch only
-owns the device memory.  Only ``decode`` exists here: the encoder belongs to training / FID preprocessing, which is out
-of scope (SURVEY.md §8).
+owns the device memory (and draws the sampling noise).  The encoder is built on the first encode call, so callers that
+only decode pay nothing for it.
 """
 from __future__ import annotations
 
@@ -55,6 +56,7 @@ class FrozenAutoencoderKL:
         self.resolution = int(ddconfig["resolution"])
         mult: Sequence[int] = ddconfig["ch_mult"]
         self.z_res = self.resolution // 2 ** (len(mult) - 1)
+        self.in_channels = int(ddconfig.get("in_channels", 3))
         self.cfg = _lib.AEConfig(int(ddconfig["ch"]), self.out_ch, int(ddconfig["num_res_blocks"]), self.z_channels,
                                  self.resolution, int(embed_dim), len(mult),
                                  (C.c_int32 * 8)(*[int(m) for m in mult]), int(max_batch), float(scale_factor))
@@ -72,6 +74,10 @@ class FrozenAutoencoderKL:
             _lib.check(self.lib.ddb_ae_create(C.byref(self.cfg), arr, len(used), C.byref(handle)))
             self.handle = handle
             del keep
+        # encoder weights stay on the host until the first encode call (see _encoder)
+        self._enc_sd = {k: v for k, v in state_dict.items()
+                        if k.startswith("encoder.") or k.startswith("quant_conv.")}
+        self._enc_built = False
 
     def __del__(self):
         h = getattr(self, "handle", None)
@@ -93,15 +99,18 @@ class FrozenAutoencoderKL:
     def requires_grad_(self, *_a, **_k):
         return self
 
+    def _check_cuda(self, t, what, shape):
+        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float32 and t.dim() == 4):
+            raise _lib.DuoDiffError(f"{what} must be a CUDA float32 tensor [B, {shape[0]}, {shape[1]}, {shape[2]}]")
+        if t.device != self.device:
+            raise _lib.DuoDiffError(f"{what} is on {t.device} but the autoencoder lives on {self.device}")
+        if tuple(t.shape[1:]) != tuple(shape):
+            raise _lib.DuoDiffError(f"{what} has shape {tuple(t.shape)}, autoencoder expects "
+                                    f"[B,{shape[0]},{shape[1]},{shape[2]}]")
+        return t.contiguous()
+
     def _check(self, z):
-        if not (z.is_cuda and z.dtype == torch.float32 and z.dim() == 4):
-            raise _lib.DuoDiffError("z must be a CUDA float32 tensor [B, z_channels, r, r]")
-        if z.device != self.device:
-            raise _lib.DuoDiffError(f"z is on {z.device} but the autoencoder lives on {self.device}")
-        if tuple(z.shape[1:]) != (self.z_channels, self.z_res, self.z_res):
-            raise _lib.DuoDiffError(f"z has shape {tuple(z.shape)}, autoencoder expects "
-                                    f"[B,{self.z_channels},{self.z_res},{self.z_res}]")
-        return z.contiguous()
+        return self._check_cuda(z, "z", (self.z_channels, self.z_res, self.z_res))
 
     def decode(self, z: torch.Tensor) -> torch.Tensor:
         """autoencoder.py:486-490: ``decoder(post_quant_conv(z / scale_factor))`` -> [B, out_ch, res, res] fp32."""
@@ -113,16 +122,73 @@ class FrozenAutoencoderKL:
         return out
 
     def forward(self, inputs, fn):  # autoencoder.py:492-500
-        if fn == "decode":
+        if fn == "encode_moments":
+            return self.encode_moments(inputs)
+        elif fn == "encode":
+            return self.encode(inputs)
+        elif fn == "decode":
             return self.decode(inputs)
-        raise NotImplementedError(f"{fn}: only 'decode' is on the sampling path")
+        raise NotImplementedError
 
     __call__ = forward
 
-    def encode(self, x):
-        raise NotImplementedError("the encoder is training / FID preprocessing (out of scope of the sampling path)")
+    # ------------------------------------------------------------------ encode side
+    def _encoder(self):
+        """Build the encoder plan on the first encode call from the ``encoder.*`` / ``quant_conv.*`` tensors kept at
+        construction (a missing key raises DuoDiffError naming it)."""
+        if self._enc_built:
+            return
+        w = self._enc_sd.get("encoder.conv_in.weight")
+        if w is not None and w.dim() == 4 and int(w.shape[1]) != self.in_channels:
+            raise _lib.DuoDiffError(f"encoder.conv_in.weight has {int(w.shape[1])} input channels, ddconfig "
+                                    f"in_channels is {self.in_channels}")
+        with torch.cuda.device(self.device):
+            keep, arr = [], (_lib.Tensor * max(len(self._enc_sd), 1))()
+            for i, (name, t) in enumerate(self._enc_sd.items()):
+                t = t.detach().to(device=self.device, dtype=torch.float32).contiguous()
+                keep.append(t)
+                arr[i] = _lib.Tensor(name.encode(), t.data_ptr(), t.numel())
+            torch.cuda.synchronize(self.device)
+            _lib.check(self.lib.ddb_ae_create_encoder(self.handle, arr, len(self._enc_sd)))
+            del keep
+        self._enc_built = True
+        self._enc_sd = {}  # packed on the device now
 
-    encode_moments = encode
+    def _check_image(self, x):
+        return self._check_cuda(x, "x", (self.in_channels, self.resolution, self.resolution))
+
+    def _moments_out(self, x):
+        return torch.empty(x.shape[0], 2 * self.embed_dim, self.z_res, self.z_res, device=x.device)
+
+    def encode_moments(self, x: torch.Tensor) -> torch.Tensor:
+        """``quant_conv(encoder(x))``: x [B, in_channels, res, res] fp32 -> moments [B, 2*embed_dim, r, r] fp32."""
+        x = self._check_image(x)
+        self._encoder()
+        out = self._moments_out(x)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.ddb_ae_encode_moments(self.handle, x.data_ptr(), x.shape[0], out.data_ptr(),
+                                                      _lib.current_stream_ptr()))
+        return out
+
+    def sample(self, moments: torch.Tensor, noise: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """``scale_factor * (mean + exp(0.5 * clamp(logvar, -30, 20)) * noise)`` with ``mean, logvar =
+        chunk(moments, 2, dim=1)``; ``noise=None`` draws ``torch.randn_like(mean)`` as the reference does."""
+        moments = self._check_cuda(moments, "moments", (2 * self.embed_dim, self.z_res, self.z_res))
+        if noise is None:
+            mean, _logvar = torch.chunk(moments, 2, dim=1)
+            noise = torch.randn_like(mean)
+        noise = self._check_cuda(noise, "noise", (self.embed_dim, self.z_res, self.z_res))
+        if noise.shape[0] != moments.shape[0]:
+            raise _lib.DuoDiffError(f"noise has batch {noise.shape[0]}, moments {moments.shape[0]}")
+        z = torch.empty(moments.shape[0], self.embed_dim, self.z_res, self.z_res, device=moments.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.ddb_ae_sample(self.handle, moments.data_ptr(), noise.data_ptr(), moments.shape[0],
+                                              z.data_ptr(), _lib.current_stream_ptr()))
+        return z
+
+    def encode(self, x: torch.Tensor, noise: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """``sample(encode_moments(x))``: x [B, in_channels, res, res] -> z [B, embed_dim, r, r] (scaled latents)."""
+        return self.sample(self.encode_moments(x), noise)
 
     # ------------------------------------------------------------------ measurement / parity hooks
     def profile_decode(self, z: torch.Tensor) -> dict:
@@ -135,14 +201,17 @@ class FrozenAutoencoderKL:
                                                       _lib.current_stream_ptr()))
         return {k: dict(ms=float(ms[i]), flops=float(fl[i])) for i, k in enumerate(self.PROF_CATEGORIES)}
 
-    def ops(self):
-        """[(name, C, H, W, is_f32)] of the launch list (C == 0: the op leaves nothing to dump)."""
+    def _op_list(self, num_ops, op_info):
         res = []
-        for i in range(self.lib.ddb_ae_num_ops(self.handle)):
+        for i in range(num_ops(self.handle)):
             name, info = C.create_string_buffer(96), (C.c_int32 * 4)()
-            _lib.check(self.lib.ddb_ae_op_info(self.handle, i, name, 96, info))
+            _lib.check(op_info(self.handle, i, name, 96, info))
             res.append((name.value.decode(), *[int(v) for v in info]))
         return res
+
+    def ops(self):
+        """[(name, C, H, W, is_f32)] of the launch list (C == 0: the op leaves nothing to dump)."""
+        return self._op_list(self.lib.ddb_ae_num_ops, self.lib.ddb_ae_op_info)
 
     def decode_debug(self, z: torch.Tensor, op_index: int):
         """(image, NCHW fp32 copy of op `op_index`'s output) for z with B <= max_batch."""
@@ -156,10 +225,38 @@ class FrozenAutoencoderKL:
         return out, dump.float().permute(0, 3, 1, 2).contiguous()
 
 
-def random_init_state_dict(ddconfig: dict = DEFAULT_DDCONFIG, embed_dim: int = 4, seed: int = 0):
+    def profile_encode(self, x: torch.Tensor) -> dict:
+        x = self._check_image(x)
+        self._encoder()
+        out = self._moments_out(x)
+        n = len(self.PROF_CATEGORIES)
+        ms, fl = (C.c_float * n)(), (C.c_double * n)()
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.ddb_ae_profile_encode(self.handle, x.data_ptr(), x.shape[0], out.data_ptr(), ms, fl,
+                                                      _lib.current_stream_ptr()))
+        return {k: dict(ms=float(ms[i]), flops=float(fl[i])) for i, k in enumerate(self.PROF_CATEGORIES)}
+
+    def encoder_ops(self):
+        """[(name, C, H, W, is_f32)] of the encoder's launch list (builds the encoder)."""
+        self._encoder()
+        return self._op_list(self.lib.ddb_ae_encoder_num_ops, self.lib.ddb_ae_encoder_op_info)
+
+    def encode_debug(self, x: torch.Tensor, op_index: int):
+        """(moments, NCHW fp32 copy of encoder op `op_index`'s output) for x with B <= max_batch."""
+        x = self._check_image(x)
+        name, c, h, w, f32 = self.encoder_ops()[op_index]
+        out = self._moments_out(x)
+        dump = torch.empty(x.shape[0], h, w, c, device=x.device, dtype=torch.float32 if f32 else torch.bfloat16)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.ddb_ae_encode_debug(self.handle, x.data_ptr(), x.shape[0], out.data_ptr(), op_index,
+                                                    dump.data_ptr(), _lib.current_stream_ptr()))
+        return out, dump.float().permute(0, 3, 1, 2).contiguous()
+
+def random_init_state_dict(ddconfig: dict = DEFAULT_DDCONFIG, embed_dim: int = 4, seed: int = 0, encoder: bool = False):
     """Decoder-side state_dict with the reference's keys and shapes (Decoder.__init__, autoencoder.py:320-412) and
     PyTorch's default Conv2d / GroupNorm initialisation -- for throughput runs, since no autoencoder checkpoint ships
-    with the reference (SURVEY.md §8d: random-init weights of the configured architecture)."""
+    with the reference (SURVEY.md §8d: random-init weights of the configured architecture).  ``encoder=True`` adds the
+    ``encoder.*`` / ``quant_conv.*`` keys (drawn after the decoder's, which stay the same)."""
     g = torch.Generator().manual_seed(seed)
     sd: Dict[str, torch.Tensor] = {}
 
@@ -197,6 +294,25 @@ def random_init_state_dict(ddconfig: dict = DEFAULT_DDCONFIG, embed_dim: int = 4
             conv(f"decoder.up.{lvl}.upsample.conv", c, c, 3)
     norm("decoder.norm_out", c)
     conv("decoder.conv_out", ddconfig["out_ch"], c, 3)
+    if not encoder:
+        return sd
+    c = ch
+    conv("encoder.conv_in", c, ddconfig.get("in_channels", 3), 3)
+    for lvl in range(len(mult)):
+        co = ch * mult[lvl]
+        for j in range(ddconfig["num_res_blocks"]):
+            res(f"encoder.down.{lvl}.block.{j}", c, co)
+            c = co
+        if lvl != len(mult) - 1:
+            conv(f"encoder.down.{lvl}.downsample.conv", c, c, 3)
+    res("encoder.mid.block_1", c, c)
+    norm("encoder.mid.attn_1.norm", c)
+    for name in ("q", "k", "v", "proj_out"):
+        conv(f"encoder.mid.attn_1.{name}", c, c, 1)
+    res("encoder.mid.block_2", c, c)
+    norm("encoder.norm_out", c)
+    conv("encoder.conv_out", 2 * zc, c, 3)
+    conv("quant_conv", 2 * embed_dim, 2 * zc, 1)
     return sd
 
 

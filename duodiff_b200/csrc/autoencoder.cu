@@ -1,6 +1,8 @@
-// KL-autoencoder decoder (FrozenAutoencoderKL.decode, models/utils/autoencoder.py:486-490 -> Decoder.forward :416-449):
-// host side of the ddb_ae_* entry points.  The decoder is compiled once into a flat list of kernel launches ("ops")
-// over a handful of NHWC bf16 buffers; ddb_ae_decode replays the list per chunk of max_batch latents.
+// KL-autoencoder decoder (FrozenAutoencoderKL.decode, models/utils/autoencoder.py:486-490 -> Decoder.forward :416-449)
+// and encoder (FrozenAutoencoderKL.encode_moments / sample / encode -> Encoder.forward): host side of the ddb_ae_*
+// entry points.  Each direction is compiled once into a flat list of kernel launches ("ops") over a handful of NHWC
+// bf16 buffers; ddb_ae_decode / ddb_ae_encode_moments replay the list per chunk of max_batch samples.  The encoder
+// plan is optional (ddb_ae_create_encoder) and reuses the decoder's activation, GroupNorm and AttnBlock workspace.
 #include <cstring>
 #include <map>
 #include <memory>
@@ -53,6 +55,16 @@ int new_buf(Buf& b, size_t bytes, bool zero = false) {
     return DDB_OK;
 }
 
+// Workspace both plans use (AttnBlock buffers): allocated by the first plan, reused by the second -- its address is
+// baked into the first plan's tensor maps, so it must never be reallocated.
+int shared_buf(Buf& b, size_t bytes, bool zero = false) {
+    if (!b) return new_buf(b, bytes, zero);
+    if (b->bytes < bytes)
+        return failf(DDB_ERR_INVALID, "autoencoder: encoder needs %zu bytes of attention workspace, the decoder has %zu",
+                     bytes, b->bytes);
+    return DDB_OK;
+}
+
 typedef std::map<std::string, const ddb_tensor*> TensorMap;
 int get_tensor(const TensorMap& tm, const std::string& name, int64_t numel, const float** out) {
     auto it = tm.find(name);
@@ -64,7 +76,7 @@ int get_tensor(const TensorMap& tm, const std::string& name, int64_t numel, cons
     return DDB_OK;
 }
 
-enum OpKind { OP_PREP, OP_CONV, OP_GN_FINALIZE, OP_GN_APPLY, OP_TRANSPOSE_V, OP_SOFTMAX };
+enum OpKind { OP_PREP, OP_CONV, OP_GN_FINALIZE, OP_GN_APPLY, OP_TRANSPOSE_V, OP_SOFTMAX, OP_IM2COL };
 enum AeCat { AC_CONV3 = 0, AC_CONV_UP, AC_CONV1, AC_ATTN_MM, AC_GN, AC_OTHER, AC_COUNT };
 
 struct Op {
@@ -113,6 +125,8 @@ struct ddb_ae {
     Buf qkv, vT, S, P, O;   // AttnBlock workspace
     Buf zero_bias;          // bias of the plain matrix products (the conv epilogue always adds one)
     std::vector<Op> ops;
+    std::vector<Op> enc_ops;  // encoder plan (empty until ddb_ae_create_encoder)
+    int enc_in_ch = 0;        // encoder in_channels (from encoder.conv_in.weight)
     float2* affine_p() const { return reinterpret_cast<float2*>(affine->p); }
 };
 
@@ -145,6 +159,16 @@ int tmap_subpixel(CUtensorMap* tm, const void* base, int N, int W, int H, int B,
     const unsigned long long str[4] = {(unsigned long long)N * 2, (unsigned long long)N * 4,
                                        (unsigned long long)W * N * 4, (unsigned long long)W * N * 8};
     const unsigned box[5] = {64, 1, (unsigned)BW, 1, (unsigned)BH};
+    return ddb_host::encode_bf16_sw128(tm, base, 5, dims, str, box);
+}
+
+// stride-2 source of the Downsample conv, NHWC [B, 2H, 2W, C] viewed as {(q, c), x, p, y, b} with source pixel
+// (2y + p, 2x + q); H, W: the output grid
+int tmap_stride2(CUtensorMap* tm, const void* base, int C, int W, int H, int B, int BW, int BH) {
+    const unsigned long long dims[5] = {2ull * C, (unsigned long long)W, 2ull, (unsigned long long)H,
+                                        (unsigned long long)B};
+    const unsigned long long str[4] = {4ull * C, 4ull * W * C, 8ull * W * C, 8ull * H * W * C};
+    const unsigned box[5] = {64, (unsigned)BW, 1, (unsigned)BH, 1};
     return ddb_host::encode_bf16_sw128(tm, base, 5, dims, str, box);
 }
 
@@ -195,7 +219,8 @@ int launch_conv(const ConvArgs& a, int BN, int epi, int num_sms, cudaStream_t st
 struct Builder {
     ddb_ae* ae;
     const TensorMap& tm;
-    int B;  // max chunk
+    int B;                 // max chunk
+    std::vector<Op>& ops;  // the plan being built (decoder or encoder)
     int part_next = 0;
 
     float2* next_part() {
@@ -258,13 +283,13 @@ struct Builder {
         f.kind = OP_GN_FINALIZE, f.cat = AC_GN, f.name = name + ".stats";
         f.part = part, f.slots = slots, f.C = C, f.cpg = C / 32, f.count = (float)((double)H * W * (C / 32));
         DDB_TRY(gn_params(key, C, &f.gamma, &f.beta));
-        ae->ops.push_back(f);
+        ops.push_back(f);
         Op a;
         a.kind = OP_GN_APPLY, a.cat = AC_GN, a.name = name;
         a.x = reinterpret_cast<const __nv_bfloat16*>(x), a.y = reinterpret_cast<__nv_bfloat16*>(y);
         a.HW = H * W, a.C = C, a.swish = swish;
         a.out = y, a.out_C = C, a.out_H = H, a.out_W = W;
-        ae->ops.push_back(a);
+        ops.push_back(a);
         return DDB_OK;
     }
 
@@ -296,7 +321,7 @@ struct Builder {
         if (res) DDB_TRY(tmap_2d(&a.tmRes, res, (size_t)B * H * W, cw->N_pad));
         o.out = out, o.out_C = cw->N_pad, o.out_H = oh, o.out_W = ow;
         o.flops_per_sample = 2.0 * (double)oh * ow * cw->N * ((subpixel ? 9.0 : (double)k * k) * C0 + C1);
-        ae->ops.push_back(o);
+        ops.push_back(o);
         return DDB_OK;
     }
 
@@ -344,18 +369,18 @@ struct Builder {
         }
         ConvW* qkv_w = cw.get();
         ae->convs.push_back(std::move(cw));
-        DDB_TRY(new_buf(ae->qkv, (size_t)B * T * 3 * C * 2));
-        DDB_TRY(new_buf(ae->vT, (size_t)B * C * T * 2));
-        DDB_TRY(new_buf(ae->S, (size_t)B * T * T * 4));
-        DDB_TRY(new_buf(ae->P, (size_t)B * T * T * 2));
-        DDB_TRY(new_buf(ae->O, (size_t)B * T * C * 2));
+        DDB_TRY(shared_buf(ae->qkv, (size_t)B * T * 3 * C * 2));
+        DDB_TRY(shared_buf(ae->vT, (size_t)B * C * T * 2));
+        DDB_TRY(shared_buf(ae->S, (size_t)B * T * T * 4));
+        DDB_TRY(shared_buf(ae->P, (size_t)B * T * T * 2));
+        DDB_TRY(shared_buf(ae->O, (size_t)B * T * C * 2));
         DDB_TRY(add_conv(name + ".qkv", AC_CONV1, qkv_w, T1, C, C, H, W, 1, false, nullptr, 0, nullptr, ae->qkv->p, nullptr));
         {
             Op t;
             t.kind = OP_TRANSPOSE_V, t.cat = AC_OTHER, t.name = name + ".vT";
             t.T = T, t.C = C, t.pitch = 3 * C, t.v_off = 2 * C;
             t.out = ae->vT->p, t.out_C = T, t.out_H = 1, t.out_W = C;
-            ae->ops.push_back(t);
+            ops.push_back(t);
         }
         {   // S[b] = q[b] k[b]^T / sqrt(C)   (autoencoder.py:174-181)
             Op o;
@@ -371,14 +396,14 @@ struct Builder {
             DDB_TRY(tmap_w(&a.tmB, reinterpret_cast<__nv_bfloat16*>(ae->qkv->p) + C, C, 3 * C, T, B, (size_t)T * 3 * C, o.BN));
             o.out = ae->S->p, o.out_C = T, o.out_H = H, o.out_W = W, o.out_f32 = 1;
             o.flops_per_sample = 2.0 * T * T * C;
-            ae->ops.push_back(o);
+            ops.push_back(o);
         }
         {
             Op s;
             s.kind = OP_SOFTMAX, s.cat = AC_OTHER, s.name = name + ".softmax";
             s.S = reinterpret_cast<const float*>(ae->S->p), s.T = T;
             s.out = ae->P->p, s.out_C = T, s.out_H = H, s.out_W = W;
-            ae->ops.push_back(s);
+            ops.push_back(s);
         }
         {   // O[b] = P[b] v[b]   (autoencoder.py:183-187)
             Op o;
@@ -389,14 +414,14 @@ struct Builder {
             DDB_TRY(tile_shape(H, W, &a.BW, &a.BH));
             a.tw = 1, a.taps = 1, a.wmode = 1;
             o.BN = pick_bn(C), o.epi = CEPI_BIAS;
-            DDB_TRY(new_buf(ae->zero_bias, (size_t)C * 4, true));
+            DDB_TRY(shared_buf(ae->zero_bias, (size_t)C * 4, true));
             a.bias = reinterpret_cast<const float*>(ae->zero_bias->p);
             DDB_TRY(tmap_act(&a.tmA0, ae->P->p, T, T, W, H, B, a.BW, a.BH));
             DDB_TRY(tmap_w(&a.tmB, ae->vT->p, T, T, C, B, (size_t)C * T, o.BN));
             DDB_TRY(tmap_2d(&a.tmOut, ae->O->p, (size_t)B * T, C));
             o.out = ae->O->p, o.out_C = C, o.out_H = H, o.out_W = W;
             o.flops_per_sample = 2.0 * T * T * C;
-            ae->ops.push_back(o);
+            ops.push_back(o);
         }
         ConvW* proj;
         DDB_TRY(pack(key + ".proj_out", C, C, 1, C, "", 0, false, &proj));
@@ -454,7 +479,7 @@ int ae_create_impl(const ddb_ae_config* cfg, const ddb_tensor* tensors, int n_te
     CUDA_TRY(cudaMemcpy(ae->pq_w->p, pw, (size_t)Cz * Cz * 4, cudaMemcpyDeviceToDevice));
     CUDA_TRY(cudaMemcpy(ae->pq_b->p, pb, (size_t)Cz * 4, cudaMemcpyDeviceToDevice));
 
-    Builder bld{ae, tm, B};
+    Builder bld{ae, tm, B, ae->ops};
     void *X = ae->act[0]->p, *Y = ae->act[1]->p, *T1 = ae->act[2]->p, *T2 = ae->act[3]->p;
     {
         Op p;
@@ -516,11 +541,151 @@ int ae_create_impl(const ddb_ae_config* cfg, const ddb_tensor* tensors, int n_te
     return DDB_OK;
 }
 
-int run_op(const ddb_ae* ae, const Op& op, int B, const float* z, float* img, cudaStream_t st) {
+// Encoder.forward + quant_conv (FrozenAutoencoderKL.encode_moments): image [B, in_ch, R, R] fp32 -> moments
+// [B, 2*embed_dim, R/2^(L-1), R/2^(L-1)] fp32.  Built on a handle whose decoder plan exists; every encoder tensor lives
+// in the decoder's activation / GroupNorm / AttnBlock workspace (checked here, true for get_autoencoder's ddconfig).
+int encoder_build(ddb_ae* ae, TensorMap& tm) {
+    const ddb_ae_config* cfg = &ae->cfg;
+    const int L = cfg->n_levels, B = ae->maxB, R = cfg->resolution, ch = cfg->ch;
+    auto it = tm.find("encoder.conv_in.weight");
+    if (it == tm.end()) return failf(DDB_ERR_MISSING_KEY, "state_dict key 'encoder.conv_in.weight' missing");
+    if (ch < 1 || it->second->numel % (9LL * ch))
+        return failf(DDB_ERR_SHAPE, "state_dict key 'encoder.conv_in.weight' has %lld elements, not ch * in_channels * 9",
+                     (long long)it->second->numel);
+    const int Cin = (int)(it->second->numel / (9LL * ch));
+    if (Cin < 1 || Cin > 7)
+        return failf(DDB_ERR_INVALID, "autoencoder: encoder in_channels %d unsupported (conv_in packs 9 * in_channels <= 64 "
+                     "im2col columns, so in_channels <= 7)", Cin);
+    if (2 * cfg->embed_dim > 8)  // the CEPI_IMG epilogue writes at most 8 fp32 channel planes
+        return failf(DDB_ERR_INVALID, "autoencoder: encoder needs 2 * embed_dim <= 8 (got embed_dim %d)", cfg->embed_dim);
+    ae->enc_in_ch = Cin;
+
+    // fit into the decoder's workspace: activations (incl. the 64-column im2col rows), affine, GroupNorm partials
+    {
+        size_t need = (size_t)R * R * 64;
+        int cmax = ch, res = R, c = ch;
+        for (int lvl = 0; lvl < L; ++lvl) {
+            const int co = ch * cfg->ch_mult[lvl], cm = c > co ? c : co;
+            if ((size_t)res * res * cm > need) need = (size_t)res * res * cm;
+            if (cm > cmax) cmax = cm;
+            c = co;
+            if (lvl != L - 1) res /= 2;
+        }
+        const size_t have = ae->act[0]->bytes / ((size_t)B * 2);
+        if (need > have)
+            return failf(DDB_ERR_INVALID, "autoencoder: encoder activations (%zu elements per sample) exceed the decoder's "
+                         "workspace (%zu)", need, have);
+        if ((size_t)B * cmax * sizeof(float2) > ae->affine->bytes)
+            return failf(DDB_ERR_INVALID, "autoencoder: encoder width %d exceeds the decoder's GroupNorm workspace", cmax);
+        const size_t slots = ((size_t)R * R) >> 7;
+        if ((size_t)B * slots * 32 * sizeof(float2) > ae->part[0]->bytes)
+            return failf(DDB_ERR_INVALID, "autoencoder: encoder GroupNorm partials exceed the decoder's workspace");
+    }
+
+    Builder bld{ae, tm, B, ae->enc_ops};
+    void *X = ae->act[0]->p, *Y = ae->act[1]->p, *T1 = ae->act[2]->p, *T2 = ae->act[3]->p;
+    {
+        Op p;
+        p.kind = OP_IM2COL, p.cat = AC_OTHER, p.name = "im2col", p.C = Cin;
+        p.out = T1, p.out_C = 64, p.out_H = R, p.out_W = R;
+        ae->enc_ops.push_back(p);
+    }
+    // conv_in as one tap over the 64 im2col columns: weight rows k = (ky*3 + kx)*Cin + c, zero-padded to K = 64
+    ConvW* cin;
+    {
+        const float *w, *b;
+        DDB_TRY(get_tensor(tm, "encoder.conv_in.weight", (int64_t)ch * Cin * 9, &w));
+        DDB_TRY(get_tensor(tm, "encoder.conv_in.bias", ch, &b));
+        std::unique_ptr<ConvW> cw(new ConvW);
+        cw->N = ch, cw->N_pad = (ch + 63) / 64 * 64, cw->ktot = 64, cw->nw = 1;
+        DDB_TRY(new_buf(cw->w, (size_t)cw->N_pad * 64 * 2, true));
+        DDB_TRY(new_buf(cw->bias, (size_t)cw->N_pad * 4, true));
+        pack_conv_kernel<<<cw->N_pad, 256>>>(w, ch, Cin, 3, 3, cw->N_pad, Cin, 64, 0, 0,
+                                             reinterpret_cast<__nv_bfloat16*>(cw->w->p));
+        LAUNCH_CHECK();
+        add_bias_kernel<<<(cw->N_pad + 255) / 256, 256>>>(b, nullptr, ch, cw->N_pad, reinterpret_cast<float*>(cw->bias->p));
+        LAUNCH_CHECK();
+        cin = cw.get();
+        ae->convs.push_back(std::move(cw));
+    }
+    int res = R, c = ch;
+    float2* px = bld.next_part();
+    int px_slots = (res * res) >> 7;
+    DDB_TRY(bld.add_conv("conv_in", AC_CONV3, cin, T1, 64, 64, res, res, 1, false, nullptr, 0, nullptr, X, px));
+    ae->enc_ops.back().flops_per_sample = 2.0 * res * res * ch * 9.0 * Cin;  // algorithmic (unpadded) work
+
+    float2* py;
+    for (int lvl = 0; lvl < L; ++lvl) {
+        const int co = ch * cfg->ch_mult[lvl];
+        for (int j = 0; j < cfg->num_res_blocks; ++j) {
+            char nm[64], key[96];
+            snprintf(nm, sizeof(nm), "down.%d.block.%d", lvl, j);
+            snprintf(key, sizeof(key), "encoder.down.%d.block.%d", lvl, j);
+            DDB_TRY(bld.add_resblock(nm, key, c, co, res, res, X, px, px_slots, T1, T2, Y, &py));
+            std::swap(X, Y), px = py;
+            c = co;
+        }
+        if (lvl != L - 1) {  // Downsample: F.pad(h, (0, 1, 0, 1)), Conv2d(c, c, 3, stride=2, padding=0)
+            char nm[64], key[96];
+            snprintf(nm, sizeof(nm), "down.%d.downsample", lvl);
+            snprintf(key, sizeof(key), "encoder.down.%d.downsample.conv", lvl);
+            ConvW* dn;
+            DDB_TRY(bld.pack(key, c, c, 3, c, "", 0, false, &dn));
+            py = bld.next_part();
+            const int ro = res / 2;
+            DDB_TRY(bld.add_conv(nm, AC_CONV3, dn, X, c, c, ro, ro, 3, false, nullptr, 0, nullptr, Y, py));
+            ConvArgs& a = ae->enc_ops.back().conv;
+            a.stride2 = 1, a.dy0 = a.dx0 = 0;
+            DDB_TRY(tmap_stride2(&a.tmA0, X, c, ro, ro, B, a.BW, a.BH));
+            std::swap(X, Y), px = py;
+            res = ro;
+            px_slots = (res * res) >> 7;
+        }
+    }
+    DDB_TRY(bld.add_resblock("mid.block_1", "encoder.mid.block_1", c, c, res, res, X, px, px_slots, T1, T2, Y, &py));
+    std::swap(X, Y), px = py;
+    DDB_TRY(bld.add_attn("mid.attn_1", "encoder.mid.attn_1", c, res, res, X, px, px_slots, T1, Y, &py));
+    std::swap(X, Y), px = py;
+    DDB_TRY(bld.add_resblock("mid.block_2", "encoder.mid.block_2", c, c, res, res, X, px, px_slots, T1, T2, Y, &py));
+    std::swap(X, Y), px = py;
+    DDB_TRY(bld.add_gn("norm_out", "encoder.norm_out", px, px_slots, X, T1, c, res, res, true));
+
+    // conv_out (c -> 2*z_channels) with quant_conv (1x1, 2*z_channels -> 2*embed_dim) folded into its weights and bias
+    // in fp32, before the bf16 rounding; the CEPI_IMG epilogue writes the moments straight into the caller's NCHW buffer
+    const int Nz = 2 * cfg->z_channels, Nm = 2 * cfg->embed_dim, K = c * 9;
+    const float *ow, *ob, *qw, *qb;
+    DDB_TRY(get_tensor(tm, "encoder.conv_out.weight", (int64_t)Nz * K, &ow));
+    DDB_TRY(get_tensor(tm, "encoder.conv_out.bias", Nz, &ob));
+    DDB_TRY(get_tensor(tm, "quant_conv.weight", (int64_t)Nm * Nz, &qw));
+    DDB_TRY(get_tensor(tm, "quant_conv.bias", Nm, &qb));
+    Buf fw, fb;
+    DDB_TRY(new_buf(fw, (size_t)Nm * K * 4));
+    DDB_TRY(new_buf(fb, (size_t)Nm * 4));
+    fold_1x1_kernel<<<Nm, 256>>>(qw, qb, ow, ob, Nm, Nz, K, reinterpret_cast<float*>(fw->p),
+                                 reinterpret_cast<float*>(fb->p));
+    LAUNCH_CHECK();
+    const ddb_tensor folded[2] = {{"moments.weight", reinterpret_cast<const float*>(fw->p), (int64_t)Nm * K},
+                                  {"moments.bias", reinterpret_cast<const float*>(fb->p), Nm}};
+    tm["moments.weight"] = &folded[0], tm["moments.bias"] = &folded[1];
+    ConvW* mo;
+    DDB_TRY(bld.pack("moments", Nm, c, 3, c, "", 0, false, &mo));
+    DDB_TRY(bld.add_conv("moments", AC_CONV3, mo, T1, c, c, res, res, 3, false, nullptr, 0, nullptr, nullptr, nullptr));
+    {
+        Op& o = ae->enc_ops.back();
+        o.epi = CEPI_IMG, o.BN = 64;
+        o.conv.img_C = Nm;
+        o.out = nullptr, o.out_C = Nm, o.out_f32 = 1;
+    }
+    CUDA_TRY(cudaDeviceSynchronize());  // the folded fp32 weights are freed on return
+    return DDB_OK;
+}
+
+// in: the plan's fp32 input (latents / image) of this chunk; out: its fp32 output (image / moments)
+int run_op(const ddb_ae* ae, const Op& op, int B, const float* in, float* out, cudaStream_t st) {
     switch (op.kind) {
         case OP_PREP: {
             const int HW = ae->zres * ae->zres, n = B * HW;
-            CUDA_TRY(ddb_host::launch_pdl(ae_prep_kernel, dim3((n + 127) / 128), dim3(128), 0, st, z,
+            CUDA_TRY(ddb_host::launch_pdl(ae_prep_kernel, dim3((n + 127) / 128), dim3(128), 0, st, in,
                                           reinterpret_cast<const float*>(ae->pq_w->p),
                                           reinterpret_cast<const float*>(ae->pq_b->p), 1.0f / ae->cfg.scale_factor, B,
                                           ae->cfg.z_channels, HW, reinterpret_cast<__nv_bfloat16*>(ae->zin->p)));
@@ -530,7 +695,7 @@ int run_op(const ddb_ae* ae, const Op& op, int B, const float* z, float* img, cu
         case OP_CONV: {
             ConvArgs a = op.conv;
             a.B = B;
-            if (op.epi == CEPI_IMG) a.img = img;
+            if (op.epi == CEPI_IMG) a.img = out;
             return launch_conv(a, op.BN, op.epi, ae->num_sms, st);
         }
         case OP_GN_FINALIZE:
@@ -567,17 +732,23 @@ int run_op(const ddb_ae* ae, const Op& op, int B, const float* z, float* img, cu
             LAUNCH_CHECK();
             return DDB_OK;
         }
+        case OP_IM2COL: {
+            const int R = ae->cfg.resolution, n = B * R * R;
+            CUDA_TRY(ddb_host::launch_pdl(ae_im2col_kernel, dim3((n + 127) / 128), dim3(128), 0, st, in, B, op.C, R, R,
+                                          reinterpret_cast<__nv_bfloat16*>(const_cast<void*>(op.out))));
+            LAUNCH_CHECK();
+            return DDB_OK;
+        }
     }
     return failf(DDB_ERR_INVALID, "bad op");
 }
 
-int decode_impl(ddb_ae* ae, const float* z, int B, float* img, cudaStream_t st, int dump_op, void* dump_dev,
-                float* ms_host, double* flops_host) {
-    const size_t zs = (size_t)ae->cfg.z_channels * ae->zres * ae->zres;
-    const size_t is = (size_t)ae->cfg.out_ch * ae->cfg.resolution * ae->cfg.resolution;
+// replay one plan per chunk of max_batch samples; in_s / out_s: fp32 elements per sample of its input / output
+int run_plan(const ddb_ae* ae, const std::vector<Op>& ops, const float* in, size_t in_s, int B, float* out,
+             size_t out_s, cudaStream_t st, int dump_op, void* dump_dev, float* ms_host, double* flops_host) {
     std::vector<cudaEvent_t> ev;
     if (ms_host) {
-        ev.resize(ae->ops.size() + 1);
+        ev.resize(ops.size() + 1);
         for (auto& e : ev) CUDA_TRY(cudaEventCreate(&e));
         for (int i = 0; i < AC_COUNT; ++i) ms_host[i] = 0.f;
         if (flops_host) for (int i = 0; i < AC_COUNT; ++i) flops_host[i] = 0.0;
@@ -585,9 +756,9 @@ int decode_impl(ddb_ae* ae, const float* z, int B, float* img, cudaStream_t st, 
     for (int b0 = 0; b0 < B; b0 += ae->maxB) {
         const int nb = (B - b0 < ae->maxB) ? B - b0 : ae->maxB;
         if (ms_host) CUDA_TRY(cudaEventRecord(ev[0], st));
-        for (size_t i = 0; i < ae->ops.size(); ++i) {
-            const Op& op = ae->ops[i];
-            DDB_TRY(run_op(ae, op, nb, z + (size_t)b0 * zs, img + (size_t)b0 * is, st));
+        for (size_t i = 0; i < ops.size(); ++i) {
+            const Op& op = ops[i];
+            DDB_TRY(run_op(ae, op, nb, in + (size_t)b0 * in_s, out + (size_t)b0 * out_s, st));
             if (ms_host) CUDA_TRY(cudaEventRecord(ev[i + 1], st));
             if ((int)i == dump_op && dump_dev && op.out && b0 == 0) {
                 const size_t bytes = (size_t)nb * op.out_C * op.out_H * op.out_W * (op.out_f32 ? 4 : 2);
@@ -596,16 +767,32 @@ int decode_impl(ddb_ae* ae, const float* z, int B, float* img, cudaStream_t st, 
         }
         if (ms_host) {
             CUDA_TRY(cudaStreamSynchronize(st));
-            for (size_t i = 0; i < ae->ops.size(); ++i) {
+            for (size_t i = 0; i < ops.size(); ++i) {
                 float ms = 0.f;
                 CUDA_TRY(cudaEventElapsedTime(&ms, ev[i], ev[i + 1]));
-                ms_host[ae->ops[i].cat] += ms;
-                if (flops_host) flops_host[ae->ops[i].cat] += ae->ops[i].flops_per_sample * nb;
+                ms_host[ops[i].cat] += ms;
+                if (flops_host) flops_host[ops[i].cat] += ops[i].flops_per_sample * nb;
             }
         }
     }
     for (auto& e : ev) cudaEventDestroy(e);
     return DDB_OK;
+}
+
+int decode_impl(ddb_ae* ae, const float* z, int B, float* img, cudaStream_t st, int dump_op, void* dump_dev,
+                float* ms_host, double* flops_host) {
+    const size_t zs = (size_t)ae->cfg.z_channels * ae->zres * ae->zres;
+    const size_t is = (size_t)ae->cfg.out_ch * ae->cfg.resolution * ae->cfg.resolution;
+    return run_plan(ae, ae->ops, z, zs, B, img, is, st, dump_op, dump_dev, ms_host, flops_host);
+}
+
+int encode_impl(ddb_ae* ae, const float* img, int B, float* moments, cudaStream_t st, int dump_op, void* dump_dev,
+                float* ms_host, double* flops_host) {
+    if (ae->enc_ops.empty())
+        return failf(DDB_ERR_INVALID, "autoencoder: no encoder on this handle (ddb_ae_create_encoder)");
+    const size_t is = (size_t)ae->enc_in_ch * ae->cfg.resolution * ae->cfg.resolution;
+    const size_t ms = (size_t)2 * ae->cfg.embed_dim * ae->zres * ae->zres;
+    return run_plan(ae, ae->enc_ops, img, is, B, moments, ms, st, dump_op, dump_dev, ms_host, flops_host);
 }
 
 }  // namespace
@@ -619,6 +806,15 @@ bool ae_set_option(const char* name, int value) {
     return false;
 }
 }  // namespace ddb_host
+
+namespace {
+int op_info(const Op& op, char* name_out, int32_t name_cap, int32_t* chw_f32_out) {
+    snprintf(name_out, name_cap, "%s", op.name.c_str());
+    chw_f32_out[0] = op.out ? op.out_C : 0, chw_f32_out[1] = op.out_H, chw_f32_out[2] = op.out_W,
+    chw_f32_out[3] = op.out_f32;
+    return DDB_OK;
+}
+}  // namespace
 
 extern "C" {
 
@@ -652,11 +848,7 @@ int32_t ddb_ae_num_ops(const ddb_ae* ae) { return ae ? (int32_t)ae->ops.size() :
 int ddb_ae_op_info(const ddb_ae* ae, int32_t i, char* name_out, int32_t name_cap, int32_t* chw_f32_out) {
     if (!ae || i < 0 || i >= (int32_t)ae->ops.size() || !name_out || !chw_f32_out)
         return failf(DDB_ERR_INVALID, "ddb_ae_op_info: bad argument");
-    const Op& op = ae->ops[i];
-    snprintf(name_out, name_cap, "%s", op.name.c_str());
-    chw_f32_out[0] = op.out ? op.out_C : 0, chw_f32_out[1] = op.out_H, chw_f32_out[2] = op.out_W,
-    chw_f32_out[3] = op.out_f32;
-    return DDB_OK;
+    return op_info(ae->ops[i], name_out, name_cap, chw_f32_out);
 }
 
 int ddb_ae_decode_debug(ddb_ae* ae, const float* z_dev, int32_t B, float* img_dev, int32_t op_index, void* dump_dev,
@@ -665,6 +857,57 @@ int ddb_ae_decode_debug(ddb_ae* ae, const float* z_dev, int32_t B, float* img_de
         return failf(DDB_ERR_INVALID, "ddb_ae_decode_debug: bad argument (B must be <= max_batch)");
     return decode_impl(ae, z_dev, B, img_dev, reinterpret_cast<cudaStream_t>(stream), op_index, dump_dev, nullptr,
                        nullptr);
+}
+
+int ddb_ae_create_encoder(ddb_ae* ae, const ddb_tensor* tensors, int32_t n_tensors) {
+    if (!ae || n_tensors < 0 || (n_tensors > 0 && !tensors)) return failf(DDB_ERR_INVALID, "ddb_ae_create_encoder: bad argument");
+    if (!ae->enc_ops.empty()) return failf(DDB_ERR_INVALID, "ddb_ae_create_encoder: the handle already has an encoder");
+    TensorMap tm;
+    for (int i = 0; i < n_tensors; ++i) tm[tensors[i].name] = &tensors[i];
+    const int r = encoder_build(ae, tm);
+    if (r != DDB_OK) ae->enc_ops.clear();  // no half-built plan: encode keeps failing with "no encoder"
+    return r;
+}
+
+int ddb_ae_encode_moments(ddb_ae* ae, const float* img_dev, int32_t B, float* moments_dev, void* stream) {
+    if (!ae || !img_dev || !moments_dev || B < 0) return failf(DDB_ERR_INVALID, "ddb_ae_encode_moments: bad argument");
+    return encode_impl(ae, img_dev, B, moments_dev, reinterpret_cast<cudaStream_t>(stream), -1, nullptr, nullptr,
+                       nullptr);
+}
+
+int ddb_ae_sample(ddb_ae* ae, const float* moments_dev, const float* noise_dev, int32_t B, float* z_dev, void* stream) {
+    if (!ae || !moments_dev || !noise_dev || !z_dev || B < 0) return failf(DDB_ERR_INVALID, "ddb_ae_sample: bad argument");
+    const int E = ae->cfg.embed_dim, HW = ae->zres * ae->zres;
+    const size_t n = (size_t)B * E * HW;
+    if (n == 0) return DDB_OK;
+    ae_sample_kernel<<<(unsigned)((n + 255) / 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+        moments_dev, noise_dev, B, E, HW, ae->cfg.scale_factor, z_dev);
+    LAUNCH_CHECK();
+    return DDB_OK;
+}
+
+int ddb_ae_profile_encode(ddb_ae* ae, const float* img_dev, int32_t B, float* moments_dev, float* ms_host,
+                          double* flops_host, void* stream) {
+    if (!ae || !img_dev || !moments_dev || !ms_host || B < 0)
+        return failf(DDB_ERR_INVALID, "ddb_ae_profile_encode: bad argument");
+    return encode_impl(ae, img_dev, B, moments_dev, reinterpret_cast<cudaStream_t>(stream), -1, nullptr, ms_host,
+                       flops_host);
+}
+
+int32_t ddb_ae_encoder_num_ops(const ddb_ae* ae) { return ae ? (int32_t)ae->enc_ops.size() : 0; }
+
+int ddb_ae_encoder_op_info(const ddb_ae* ae, int32_t i, char* name_out, int32_t name_cap, int32_t* chw_f32_out) {
+    if (!ae || i < 0 || i >= (int32_t)ae->enc_ops.size() || !name_out || !chw_f32_out)
+        return failf(DDB_ERR_INVALID, "ddb_ae_encoder_op_info: bad argument");
+    return op_info(ae->enc_ops[i], name_out, name_cap, chw_f32_out);
+}
+
+int ddb_ae_encode_debug(ddb_ae* ae, const float* img_dev, int32_t B, float* moments_dev, int32_t op_index,
+                        void* dump_dev, void* stream) {
+    if (!ae || !img_dev || !moments_dev || B < 0 || B > ae->maxB)
+        return failf(DDB_ERR_INVALID, "ddb_ae_encode_debug: bad argument (B must be <= max_batch)");
+    return encode_impl(ae, img_dev, B, moments_dev, reinterpret_cast<cudaStream_t>(stream), op_index, dump_dev,
+                       nullptr, nullptr);
 }
 
 }  // extern "C"

@@ -20,6 +20,10 @@
 // low-resolution source, so the layer is four 2x2-tap convolutions with pre-summed weights (2.25x fewer FLOPs); each
 // class stores its tile through a 5-D tensor map {n, px, x, py, b*H + y} of the high-resolution output.
 //
+// The encoder's Downsample (F.pad(h, (0,1,0,1)) then a 3x3 stride-2 convolution) is the same idea on the load side:
+// the tile walk stays on the half-resolution output grid and the source is read through a 5-D tensor map
+// {(q, c), x, p, y, b} with source pixel (2y + p, 2x + q), so every tap is again ONE box (ConvArgs::stride2).
+//
 // Roles (384 threads, 1 CTA / SM, persistent over tiles): warp 0 TMA producer, warp 1 MMA issuer, warp 2 TMEM
 // allocator, warps 4-11 epilogue (two warpgroups, 64-column chunks, double-buffered TMEM accumulator).
 // The epilogue can also emit the GroupNorm statistics of the NEXT layer: per (tile, group) sums of x and x^2 of the
@@ -48,6 +52,10 @@ struct ConvArgs {
     int BW, BH;              // pixel tile: BH rows x BW columns = 128 pixels
     int wmode;               // 0 one weight set, 1 one per sample (batched matmul), 2 one per sub-pixel class
     int subpixel;            // fused nearest-2x upsample: 4 parity classes, taps 2x2, dy0/dx0 derived per class
+    int stride2;             // stride-2 3x3 conv over a 2H x 2W source (Downsample); tmA0 is then the 5-D view
+                             // {2*C0 (q*C0 + c), W, 2 (p), H, B} of it and tap (ky, kx) is one box at
+                             // (kx&1, x + (kx>>1), ky&1, y + (ky>>1)); the zero fill past the right / bottom edge is
+                             // F.pad(h, (0, 1, 0, 1))
     const float* bias;       // [N] or nullptr
     float2* gn_part;         // optional [B][slots][32] (sum, sum of squares) of the stored values per GroupNorm group
     int cpg;                 // output channels per group (N / 32)
@@ -167,10 +175,18 @@ __global__ void __launch_bounds__(384, 1) conv_igemm_kernel(const __grid_constan
                     uint8_t* dA = sA + stage * (MT * Cfg::A_BYTES);
                     if (kb < nkb0) {
                         const int ty = tap / a.tw, tx = tap - ty * a.tw;
+                        if (a.stride2) {
 #pragma unroll
-                        for (int mt = 0; mt < MT; ++mt)
-                            tma_load_4d(dA + mt * Cfg::A_BYTES, &a.tmA0, &full_bar[stage], cc * Cfg::BK,
-                                        tx0[mt] + dx0 + tx, ty0[mt] + dy0 + ty, tb[mt]);
+                            for (int mt = 0; mt < MT; ++mt)
+                                tma_load_5d(dA + mt * Cfg::A_BYTES, &a.tmA0, &full_bar[stage],
+                                            cc * Cfg::BK + (tx & 1) * a.C0, tx0[mt] + (tx >> 1), ty & 1,
+                                            ty0[mt] + (ty >> 1), tb[mt]);
+                        } else {
+#pragma unroll
+                            for (int mt = 0; mt < MT; ++mt)
+                                tma_load_4d(dA + mt * Cfg::A_BYTES, &a.tmA0, &full_bar[stage], cc * Cfg::BK,
+                                            tx0[mt] + dx0 + tx, ty0[mt] + dy0 + ty, tb[mt]);
+                        }
                         if (++cc == cpk) cc = 0, ++tap;
                     } else {
 #pragma unroll
@@ -389,6 +405,7 @@ __global__ void __launch_bounds__(384, 1) conv_igemm_kernel(const __grid_constan
                             reinterpret_cast<float4*>(dst)[j] = o;
                         }
                     } else {  // CEPI_IMG: consecutive lanes are consecutive pixels of one channel plane
+                        // (img_C <= 8: out_ch of the decoder, 2 * embed_dim moments of the encoder)
                         const size_t plane = (size_t)a.H * a.W;
                         float* dst = a.img + (size_t)b * a.img_C * plane + p0 + row_in_tile;
 #pragma unroll
@@ -439,6 +456,71 @@ __global__ void ae_prep_kernel(const float* __restrict__ z, const float* __restr
         o.x = pack_bf16(v[0], v[1]), o.y = pack_bf16(v[2], v[3]), o.z = pack_bf16(v[4], v[5]),
         o.w = pack_bf16(v[6], v[7]);
         dst[j] = o;
+    }
+}
+
+// Encoder conv_in over the caller's image x [B, Cin, H, W] fp32 (Cin <= 7): im2col rows [B*H*W, 64] bf16 with column
+// (ky*3 + kx)*Cin + c = x[b, c, y + ky - 1, x + kx - 1] (zero outside the image, zero in columns >= 9*Cin), so that
+// conv_in runs as a one-tap convolution with K = 64 instead of nine taps over 64 zero-padded channels.
+__global__ void ae_im2col_kernel(const float* __restrict__ img, int B, int Cin, int H, int W,
+                                 __nv_bfloat16* __restrict__ out) {
+    pdl_launch_dependents();
+    pdl_wait();
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;  // pixel over B*H*W
+    if (p >= B * H * W) return;
+    const int b = p / (H * W), i = p % (H * W), y = i / W, x = i % W;
+    const float* src = img + (size_t)b * Cin * H * W;
+    float v[64];  // compile-time indices only: stays in registers
+    int t = 0, c = 0, ky = 0, kx = 0;
+#pragma unroll
+    for (int k = 0; k < 64; ++k) {
+        const int yy = y + ky - 1, xx = x + kx - 1;
+        v[k] = (t < 9 && yy >= 0 && yy < H && xx >= 0 && xx < W) ? src[((size_t)c * H + yy) * W + xx] : 0.f;
+        if (++c == Cin) {
+            c = 0, ++t;
+            if (++kx == 3) kx = 0, ++ky;
+        }
+    }
+    uint4* dst = reinterpret_cast<uint4*>(out + (size_t)p * 64);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        uint4 o;
+        o.x = pack_bf16(v[j * 8 + 0], v[j * 8 + 1]), o.y = pack_bf16(v[j * 8 + 2], v[j * 8 + 3]);
+        o.z = pack_bf16(v[j * 8 + 4], v[j * 8 + 5]), o.w = pack_bf16(v[j * 8 + 6], v[j * 8 + 7]);
+        dst[j] = o;
+    }
+}
+
+// DiagonalGaussian sample of FrozenAutoencoderKL.sample: moments [B, 2E, HW] fp32 (mean | logvar), noise [B, E, HW]
+//   z = scale * (mean + exp(0.5 * clamp(logvar, -30, 20)) * noise)
+// in torch's operation order, without FMA contraction.
+__global__ void ae_sample_kernel(const float* __restrict__ moments, const float* __restrict__ noise, int B, int E,
+                                 int HW, float scale, float* __restrict__ z) {
+    const size_t n = (size_t)B * E * HW;
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const size_t b = i / ((size_t)E * HW), r = i % ((size_t)E * HW);
+    const float mean = moments[b * 2 * E * HW + r];
+    const float logvar = fminf(fmaxf(moments[b * 2 * E * HW + (size_t)E * HW + r], -30.f), 20.f);
+    const float stdv = expf(__fmul_rn(0.5f, logvar));
+    z[i] = __fmul_rn(scale, __fadd_rn(mean, __fmul_rn(stdv, noise[i])));
+}
+
+// quant_conv (1x1, Nj -> No) folded into the preceding conv (w [Nj, K], b [Nj]) in fp32:
+//   w'[o, k] = sum_j wq[o, j] w[j, k],  b'[o] = bq[o] + sum_j wq[o, j] b[j]
+__global__ void fold_1x1_kernel(const float* __restrict__ wq, const float* __restrict__ bq,
+                                const float* __restrict__ w, const float* __restrict__ b, int No, int Nj, int K,
+                                float* __restrict__ w_out, float* __restrict__ b_out) {
+    const int o = blockIdx.x;
+    for (int k = threadIdx.x; k < K; k += blockDim.x) {
+        float acc = 0.f;
+        for (int j = 0; j < Nj; ++j) acc = fmaf(wq[o * Nj + j], w[(size_t)j * K + k], acc);
+        w_out[(size_t)o * K + k] = acc;
+    }
+    if (threadIdx.x == 0) {
+        float acc = bq[o];
+        for (int j = 0; j < Nj; ++j) acc = fmaf(wq[o * Nj + j], b[j], acc);
+        b_out[o] = acc;
     }
 }
 

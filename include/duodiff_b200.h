@@ -174,7 +174,8 @@ typedef struct {
     float scale_factor;      /* 0.18215 */
 } ddb_ae_config;
 typedef struct ddb_ae ddb_ae;
-/* tensors: the FrozenAutoencoderKL state_dict (keys `post_quant_conv.*`, `decoder.*`; encoder keys are ignored). */
+/* tensors: the FrozenAutoencoderKL state_dict (keys `post_quant_conv.*`, `decoder.*`; encoder keys are ignored here,
+ * see ddb_ae_create_encoder). */
 int ddb_ae_create(const ddb_ae_config* cfg, const ddb_tensor* tensors, int32_t n_tensors, ddb_ae** out);
 void ddb_ae_destroy(ddb_ae* ae);
 /* FrozenAutoencoderKL.decode(z) (models/utils/autoencoder.py:486-490):
@@ -192,6 +193,28 @@ int32_t ddb_ae_num_ops(const ddb_ae* ae);
 int ddb_ae_op_info(const ddb_ae* ae, int32_t i, char* name_out, int32_t name_cap, int32_t* info_out);
 int ddb_ae_decode_debug(ddb_ae* ae, const float* z_dev, int32_t B, float* img_dev, int32_t op_index, void* dump_dev,
                         void* stream);
+
+/* ---- KL-autoencoder encode: image -> latent (FrozenAutoencoderKL.encode_moments / sample / encode) ----
+ * ddb_ae_create_encoder adds the Encoder + quant_conv plan to a handle made by ddb_ae_create, from the keys
+ * `encoder.*` and `quant_conv.*` (other keys are ignored; a missing one gives DDB_ERR_MISSING_KEY).  in_channels
+ * (<= 7) is read from encoder.conv_in.weight.  The encoder shares the decoder's workspace and plays no part in
+ * decode; both plans may be used on one handle, one call at a time. */
+int ddb_ae_create_encoder(ddb_ae* ae, const ddb_tensor* tensors, int32_t n_tensors);
+/* encode_moments(x) = quant_conv(encoder(x)):
+ *   img_dev [B, in_channels, resolution, resolution] f32 -> moments_dev [B, 2*embed_dim, r, r] f32 (mean | logvar),
+ *   processed in chunks of max_batch. */
+int ddb_ae_encode_moments(ddb_ae* ae, const float* img_dev, int32_t B, float* moments_dev, void* stream);
+/* sample(moments) with caller-supplied standard-normal noise_dev [B, embed_dim, r, r]:
+ *   z_dev = scale_factor * (mean + exp(0.5 * clamp(logvar, -30, 20)) * noise)   [B, embed_dim, r, r] f32. */
+int ddb_ae_sample(ddb_ae* ae, const float* moments_dev, const float* noise_dev, int32_t B, float* z_dev, void* stream);
+/* Profile / parity hooks of the encoder plan, as for decode (same DDB_AE_PROF_CATEGORIES; the stride-2 Downsample
+ * convolutions count as conv3x3, the im2col prep of conv_in as other). */
+int ddb_ae_profile_encode(ddb_ae* ae, const float* img_dev, int32_t B, float* moments_dev, float* ms_host,
+                          double* flops_host, void* stream);
+int32_t ddb_ae_encoder_num_ops(const ddb_ae* ae);
+int ddb_ae_encoder_op_info(const ddb_ae* ae, int32_t i, char* name_out, int32_t name_cap, int32_t* info_out);
+int ddb_ae_encode_debug(ddb_ae* ae, const float* img_dev, int32_t B, float* moments_dev, int32_t op_index,
+                        void* dump_dev, void* stream);
 
 /* ---- single-operator entry points (used by the parity tests; same kernels as the model path) ---- */
 /* out[M,N] = epi([A0|A1] W^T); bf16 row-major operands.  epi: 0 bias, 1 LN-fold, 2 LN-fold+GELU, 3 bias+residual.
