@@ -6,6 +6,7 @@ signature, logs and CLI flags (eesampler.py:40-89,114-134).  The loop runs insid
 """
 from __future__ import annotations
 
+import functools
 import time
 from argparse import ArgumentParser
 from pathlib import Path
@@ -14,6 +15,7 @@ import numpy as np
 import torch
 
 from . import _io
+from . import distributed as D
 from .autoencoder import get_autoencoder
 from .ddpm import cached_sampler
 from .sampler import _pick_device, draw_labels
@@ -86,33 +88,48 @@ def get_args(argv=None):
 
 
 def main(argv=None):
+    """The reference's CLI.  Under `torchrun --nproc-per-node N` each rank samples its shard of the --batch_size
+    images (duodiff_b200.distributed) and rank 0 writes exactly the files a single process writes."""
     args = get_args(argv)
     out_dir = Path(args.output_folder)
-    out_dir.mkdir(parents=True, exist_ok=True)
+    if D.env_rank_world()[0] == 0:
+        out_dir.mkdir(parents=True, exist_ok=True)
     if not torch.cuda.is_available():
         raise RuntimeError("duodiff_b200.eesampler needs a B200 (sm_100) GPU; there is no CPU path")
-    device = torch.device("cuda:0")
-    print(f"Using device {device}")
-    cfg = _io.load_config(args.config_path)
-    mp = cfg["model_params"]
-    model = EarlyExitUViT(UViT(**_io.uvit_kwargs(cfg), max_batch=args.batch_size), mp["classifier_type"])
-    _io.load_checkpoint_into(model, args.checkpoint_path)
-    model = model.eval().to(device)
-    _io.seed_everything(args.seed)
-    y = None
-    if args.class_id is not None:
-        y = draw_labels(args.batch_size, mp.get("num_classes", -1)).to(device)
-    autoencoder = None
-    if "autoencoder" in cfg:  # eesampler.py:184-189
-        autoencoder = get_autoencoder(cfg["autoencoder"]["autoencoder_checkpoint_path"])
-    tic = time.time()
-    samples, err_log, idx_log = get_samples(
-        model=model, batch_size=args.batch_size, seed=args.seed, num_channels=mp["in_chans"],
-        sample_height=mp["img_size"], sample_width=mp["img_size"], threshold=args.threshold, depth=mp["depth"], y=y,
-        autoencoder=autoencoder)
-    tac = time.time()
-    dump_statistics(tac - tic, err_log, idx_log, out_dir)
-    dump_samples(samples, out_dir)
+    with D.cli_process_group() as (rank, world, device):
+        print(f"Using device {device}")
+        cfg = _io.load_config(args.config_path)
+        mp = cfg["model_params"]
+        lo, hi = D.shard_bounds(args.batch_size, rank, world)
+        model = autoencoder = None
+        if hi > lo:  # a rank with an empty shard (more ranks than images) builds nothing
+            model = EarlyExitUViT(UViT(**_io.uvit_kwargs(cfg), max_batch=hi - lo), mp["classifier_type"])
+            _io.load_checkpoint_into(model, args.checkpoint_path)
+            model = model.eval().to(device)
+        _io.seed_everything(args.seed)
+        y = None
+        if args.class_id is not None:
+            y = draw_labels(args.batch_size, mp.get("num_classes", -1)).to(device)
+        if "autoencoder" in cfg and hi > lo:  # eesampler.py:184-189
+            autoencoder = get_autoencoder(cfg["autoencoder"]["autoencoder_checkpoint_path"])
+        D.barrier()  # every rank has loaded its model: the clock starts together
+        tic = time.time()
+        local = D.run_shard(
+            functools.partial(get_samples, model=model), args.batch_size,
+            shape=(mp["in_chans"], mp["img_size"], mp["img_size"]), seed=args.seed, y=y,
+            num_channels=mp["in_chans"], sample_height=mp["img_size"], sample_width=mp["img_size"],
+            threshold=args.threshold, depth=mp["depth"], autoencoder=autoencoder)
+        D.barrier()  # every shard is done: what follows is the gather alone
+        t_gather = time.time()
+        result = D.gather_to_rank0(local, args.batch_size, D.EESAMPLER_OUTPUTS)
+        tac = time.time()
+        if rank != 0:
+            return
+        if world > 1:
+            print(f"Gathered {args.batch_size} samples from {world} ranks in {tac - t_gather:.3f} s")
+        samples, err_log, idx_log = result
+        dump_statistics(tac - tic, err_log, idx_log, out_dir)
+        dump_samples(samples, out_dir)
 
 
 if __name__ == "__main__":

@@ -8,6 +8,7 @@ update — runs inside libduodiff_b200.so as CUDA-graph replays of hand-written 
 """
 from __future__ import annotations
 
+import functools
 import time
 from argparse import ArgumentParser
 from pathlib import Path
@@ -17,6 +18,7 @@ import numpy as np
 import torch
 
 from . import _io
+from . import distributed as D
 from .autoencoder import get_autoencoder
 from .ddpm import RULES, cached_sampler, ddim_timesteps
 from .uvit import UViT
@@ -196,37 +198,54 @@ def _build(config_path, checkpoint_path, batch_size, device):
 
 
 def main(argv=None):
+    """The reference's CLI.  Under `torchrun --nproc-per-node N` each rank samples its shard of the --batch_size
+    images (duodiff_b200.distributed) and rank 0 writes exactly the files a single process writes."""
     args = get_args(argv)
     out_dir = Path(args.output_folder)
-    out_dir.mkdir(parents=True, exist_ok=True)
+    if D.env_rank_world()[0] == 0:
+        out_dir.mkdir(parents=True, exist_ok=True)
     if not torch.cuda.is_available():
         raise RuntimeError("duodiff_b200.sampler needs a B200 (sm_100) GPU; there is no CPU path")
-    device = torch.device("cuda:0")
-    print(f"Using device {device}")
-    model, cfg = _build(args.config_path, args.checkpoint_path, args.batch_size, device)
-    late = None
-    if args.checkpoint_path_late:
-        late, cfg = _build(args.config_path_late, args.checkpoint_path_late, args.batch_size, device)
-    mp = cfg["model_params"]
-    _io.seed_everything(args.seed)
-    y = None
-    if args.class_id is not None:
-        y = draw_labels(args.batch_size, mp.get("num_classes", -1)).to(device)
-    autoencoder = None
-    if "autoencoder" in cfg:  # sampler.py:320-325
-        autoencoder = get_autoencoder(cfg["autoencoder"]["autoencoder_checkpoint_path"])
-    tic = time.time()
-    samples, inter = get_samples(
-        model=model, batch_size=args.batch_size, postprocessing=_BY_NAME[args.parametrization], seed=args.seed,
-        num_channels=mp["in_chans"], sample_height=mp["img_size"], sample_width=mp["img_size"],
-        use_ddim=args.use_ddim, ddim_steps=args.ddim_steps, ddim_eta=args.ddim_eta, y=y, autoencoder=autoencoder,
-        late_model=late, t_switch=args.t_switch, timesteps_save=args.timesteps_save)
-    tac = time.time()
-    dump_statistics(tac - tic, out_dir)
-    dump_samples(samples, out_dir)
-    if args.timesteps_save:
-        for ts, s in zip(args.timesteps_save, inter):
-            dump_samples(s, out_dir, ts)
+    with D.cli_process_group() as (rank, world, device):
+        print(f"Using device {device}")
+        lo, hi = D.shard_bounds(args.batch_size, rank, world)
+        model = late = autoencoder = None
+        if hi > lo:  # a rank with an empty shard (more ranks than images) builds nothing
+            model, cfg = _build(args.config_path, args.checkpoint_path, hi - lo, device)
+            if args.checkpoint_path_late:
+                late, cfg = _build(args.config_path_late, args.checkpoint_path_late, hi - lo, device)
+        else:
+            cfg = _io.load_config(args.config_path_late if args.checkpoint_path_late else args.config_path)
+        mp = cfg["model_params"]
+        _io.seed_everything(args.seed)
+        y = None
+        if args.class_id is not None:
+            y = draw_labels(args.batch_size, mp.get("num_classes", -1)).to(device)
+        if "autoencoder" in cfg and hi > lo:  # sampler.py:320-325
+            autoencoder = get_autoencoder(cfg["autoencoder"]["autoencoder_checkpoint_path"])
+        D.barrier()  # every rank has loaded its models: the clock starts together
+        tic = time.time()
+        local = D.run_shard(
+            functools.partial(get_samples, model=model), args.batch_size,
+            shape=(mp["in_chans"], mp["img_size"], mp["img_size"]), seed=args.seed, y=y,
+            postprocessing=_BY_NAME[args.parametrization], num_channels=mp["in_chans"],
+            sample_height=mp["img_size"], sample_width=mp["img_size"], use_ddim=args.use_ddim,
+            ddim_steps=args.ddim_steps, ddim_eta=args.ddim_eta, autoencoder=autoencoder, late_model=late,
+            t_switch=args.t_switch, timesteps_save=args.timesteps_save)
+        D.barrier()  # every shard is done: what follows is the gather alone
+        t_gather = time.time()
+        result = D.gather_to_rank0(local, args.batch_size, D.SAMPLER_OUTPUTS)
+        tac = time.time()
+        if rank != 0:
+            return
+        if world > 1:
+            print(f"Gathered {args.batch_size} samples from {world} ranks in {tac - t_gather:.3f} s")
+        samples, inter = result
+        dump_statistics(tac - tic, out_dir)
+        dump_samples(samples, out_dir)
+        if args.timesteps_save:
+            for ts, s in zip(args.timesteps_save, inter):
+                dump_samples(s, out_dir, ts)
 
 
 if __name__ == "__main__":
