@@ -50,6 +50,7 @@ _SIGS = {
                                      C.POINTER(_P)]),
     "ddb_sampler_destroy": (None, [_P]),
     "ddb_sampler_set_noise_offset": (C.c_int, [_P, C.c_uint64]),
+    "ddb_sampler_set_guidance": (C.c_int, [_P, C.c_float, C.c_int64]),
     "ddb_sampler_profile_step": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P]),
     "ddb_sampler_run": (C.c_int, [_P, _P, _P, _P, C.c_uint64, C.c_int32, C.c_int32, _P, _P, _P, _P, C.c_int32, _P]),
     "ddb_sampler_run_list": (C.c_int, [_P, _P, _P, _P, C.c_uint64, _P, _P, C.c_int32, _P, _P, C.c_int32, _P]),

@@ -5,6 +5,7 @@
 
 #include <algorithm>
 #include <atomic>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
@@ -1033,12 +1034,13 @@ struct EeCompact {
 struct StepFuse {
     TailArgs tail;
 };
-static int launch_patch_gather(const ddb_model* m, const float* x, int B, cudaStream_t st) {
+// row0: first row of the patch matrix written (the guided sampler gathers x into rows [0, B) and [B, 2B))
+static int launch_patch_gather(const ddb_model* m, const float* x, int B, cudaStream_t st, int row0 = 0) {
     const ddb_uvit_config& c = m->cfg;
     const size_t n_thr = (size_t)B * c.in_chans * c.img_size * (c.img_size / c.patch_size);
     CUDA_TRY(launch_pdl(patch_gather_kernel, dim3((unsigned)((n_thr + 255) / 256)), dim3(256), 0, st, x,
-                        m->a_patch->as<__nv_bfloat16>(), B, (int)c.in_chans, (int)c.img_size, (int)c.img_size,
-                        (int)c.patch_size));
+                        m->a_patch->as<__nv_bfloat16>() + (size_t)row0 * m->Np * 128, B, (int)c.in_chans,
+                        (int)c.img_size, (int)c.img_size, (int)c.patch_size));
     LAUNCH_CHECK();
     return DDB_OK;
 }
@@ -1064,11 +1066,23 @@ static int launch_token_extras(const ddb_model* m, const float* t_vec, const int
     LAUNCH_CHECK();
     return DDB_OK;
 }
+// B: rows of the forward; a guided tail runs one CTA per guided sample (ta.B = B / 2) and band
 static int launch_step_tail(const ddb_model* m, const TailArgs& ta, int B, cudaStream_t st) {
     const int C = m->cfg.in_chans, H = m->cfg.img_size, W = m->cfg.img_size;
-    const dim3 grid(B * (H / CONV_BAND));
+    const dim3 grid((ta.guide ? ta.B : B) * (H / CONV_BAND));
     ProfScope ps(PC_TAIL);
-    if (C == 3 && W == 64)
+    if (ta.guide) {
+        if (C == 3 && W == 64)
+            CUDA_TRY(launch_pdl(step_tail_kernel<3, 64, true>, grid, dim3(256), 0, st, ta));
+        else if (C == 3 && W == 32)
+            CUDA_TRY(launch_pdl(step_tail_kernel<3, 32, true>, grid, dim3(256), 0, st, ta));
+        else if (C == 4 && W == 32)
+            CUDA_TRY(launch_pdl(step_tail_kernel<4, 32, true>, grid, dim3(256), 0, st, ta));
+        else if (C == 4 && W == 64)
+            CUDA_TRY(launch_pdl(step_tail_kernel<4, 64, true>, grid, dim3(256), 0, st, ta));
+        else
+            return fail(DDB_ERR_INVALID, "sample shape [%d,%d,%d] unsupported by the guided step tail", C, H, W);
+    } else if (C == 3 && W == 64)
         CUDA_TRY(launch_pdl(step_tail_kernel<3, 64>, grid, dim3(256), 0, st, ta));
     else if (C == 3 && W == 32)
         CUDA_TRY(launch_pdl(step_tail_kernel<3, 32>, grid, dim3(256), 0, st, ta));
@@ -1433,9 +1447,15 @@ struct ddb_sampler {
     long long graph_nodes[2] = {0, 0};
     struct Key {
         const void* z_all = nullptr;
-        int has_y = 0, epoch = -1;
-        bool operator==(const Key& o) const { return z_all == o.z_all && has_y == o.has_y && epoch == o.epoch; }
+        int has_y = 0, epoch = -1, guide = 0;
+        float scale = 0.f;
+        bool operator==(const Key& o) const {
+            return z_all == o.z_all && has_y == o.has_y && epoch == o.epoch && guide == o.guide && scale == o.scale;
+        }
     } graph_key[2];
+    // classifier-free guidance (ddb_sampler_set_guidance): every forward runs on 2B rows, y_buf holds [y ; null...]
+    int guide = 0;
+    float cfg_scale = 0.f;
     bool early_exit() const { return ee_mode >= 0 && early->cfg.early_exit; }
     // every step ends in step_tail_kernel, which also prepares the head of the next step (plain backbones always;
     // early exit in compaction mode on the CTA-pair path, option "ee_fuse")
@@ -1475,7 +1495,7 @@ static void tail_target(TailTarget& tg, const ddb_model* m) {
 //   early exit, simulate (or ee_fuse = 0):  fill_t -> EarlyExitUViT forward + selection -> ddpm_step -> next_t
 static int sampler_step(ddb_sampler* s, ddb_model* m, float* x, bool has_y, const float* z_all, float* eps_save,
                         float* x_save, cudaStream_t st) {
-    const int B = s->B;
+    const int B = s->B;  // samples; a guided forward runs on 2B rows
     const int64_t* y = has_y ? s->y_buf->as<int64_t>() : nullptr;
     const bool ee_on = s->early_exit() && m->cfg.early_exit;
     if (ee_on && !s->fused()) {
@@ -1516,6 +1536,8 @@ static int sampler_step(ddb_sampler* s, ddb_model* m, float* x, bool has_y, cons
     ta.n = s->n, ta.H = m->cfg.img_size, ta.W = m->cfg.img_size, ta.mode = s->step_mode;
     tail_target(ta.tgt[0], s->early);
     tail_target(ta.tgt[1], s->late ? s->late : s->early);
+    ta.guide = s->guide, ta.scale = s->cfg_scale, ta.B = B;
+    if (s->guide) return forward_impl(m, x, nullptr, y, 2 * B, nullptr, false, st, nullptr, &f);
     if (ee_on) {
         // early exit with compaction: the same fused step; the tail picks every sample's conv weights by its exit layer
         EeCompact cp{s->ee_threshold, m->exit_idx->as<int32_t>(), s->t_dev->as<int>(), s->exit_log->as<int32_t>(),
@@ -1728,6 +1750,34 @@ void ddb_sampler_destroy(ddb_sampler* s) {
         if (s->graph[i]) cudaGraphExecDestroy(s->graph[i]);
     delete s;
 }
+int ddb_sampler_set_guidance(ddb_sampler* s, float scale, int64_t null_label) {
+    if (!s) return fail(DDB_ERR_INVALID, "null argument");
+    if (!std::isfinite(scale)) return fail(DDB_ERR_INVALID, "guidance scale %g is not finite", (double)scale);
+    if (s->ee_mode >= 0)
+        return fail(DDB_ERR_INVALID, "guidance is not supported with early exit (the conditional and unconditional "
+                                     "rows would leave at different layers)");
+    for (const ddb_model* m : {s->early, s->late}) {
+        if (!m) continue;
+        if (m->cfg.num_classes <= 0) return fail(DDB_ERR_INVALID, "guidance needs class-conditional models");
+        if (null_label < 0 || null_label >= m->cfg.num_classes)
+            return fail(DDB_ERR_INVALID, "null label %lld outside [0, %d)", (long long)null_label, m->cfg.num_classes);
+        if (m->cfg.max_batch < 2 * s->B)
+            return fail(DDB_ERR_INVALID, "guidance runs the forward on 2B = %d rows but a model has max_batch = %d",
+                        2 * s->B, m->cfg.max_batch);
+    }
+    // captured steps bake in the label buffer and the scale: they are captured again on the next run
+    CUDA_TRY(cudaDeviceSynchronize());
+    for (int i = 0; i < 2; ++i)
+        if (s->graph[i]) cudaGraphExecDestroy(s->graph[i]), s->graph[i] = nullptr;
+    // labels [y ; null x B]: the run copies y into the first half, the null half is written once here
+    Buf y2;
+    DDB_TRY(new_buf(y2, (size_t)2 * s->B * 8));
+    std::vector<int64_t> nulls((size_t)s->B, null_label);
+    CUDA_TRY(cudaMemcpy(y2->as<int64_t>() + s->B, nulls.data(), (size_t)s->B * 8, cudaMemcpyHostToDevice));
+    s->y_buf = std::move(y2);
+    s->guide = 1, s->cfg_scale = scale;
+    return DDB_OK;
+}
 int ddb_sampler_set_noise_offset(ddb_sampler* s, uint64_t first_row) {
     if (!s) return fail(DDB_ERR_INVALID, "null argument");
     s->noise_row0 = first_row;
@@ -1776,10 +1826,13 @@ static int sampler_run_impl(ddb_sampler* s, float* x_dev, const int64_t* y_dev, 
         CUDA_TRY(cudaMemcpyAsync(xw, x_dev, s->n * 4, cudaMemcpyDeviceToDevice, st));
     }
     if (s->fused()) {
-        // head of the first step (every later step's head is written by its predecessor's tail kernel)
+        // head of the first step (every later step's head is written by its predecessor's tail kernel); guided: x in
+        // both halves of the patch matrix, token rows for [y ; null]
         ddb_model* m0 = late[0] ? s->late : s->early;
         DDB_TRY(launch_patch_gather(m0, xw, s->B, st));
-        DDB_TRY(launch_token_extras(m0, nullptr, s->t_dev->as<int>(), has_y ? s->y_buf->as<int64_t>() : nullptr, s->B, st));
+        if (s->guide) DDB_TRY(launch_patch_gather(m0, xw, s->B, st, s->B));
+        DDB_TRY(launch_token_extras(m0, nullptr, s->t_dev->as<int>(), has_y ? s->y_buf->as<int64_t>() : nullptr,
+                                    s->guide ? 2 * s->B : s->B, st));
     }
     if (!use_graph) {
         for (int k = 0; k < n; ++k) {
@@ -1791,6 +1844,7 @@ static int sampler_run_impl(ddb_sampler* s, float* x_dev, const int64_t* y_dev, 
         // ---- one captured step per backbone
         ddb_sampler::Key key;
         key.z_all = z_all_dev, key.has_y = has_y ? 1 : 0, key.epoch = g_option_epoch.load();
+        key.guide = s->guide, key.scale = s->cfg_scale;
         for (int which = 0; which < 2; ++which) {
             ddb_model* m = which == 0 ? s->early : s->late;
             if (!m) continue;

@@ -504,13 +504,21 @@ struct TailArgs {
     const float* grp_b;
     int depth;
     TailTarget tgt[2];     // [0] early backbone, [1] late backbone
+    // classifier-free guidance: the forward ran on 2B rows (row b conditional, row b + B unconditional); the tail
+    // combines them into eps = c + scale * (c - u) per guided sample b < B and prepares the head of both rows
+    int guide;             // 0 / 1; selects the G = true instantiation on the host
+    float scale;
+    int B;                 // guided samples (x, noise and traces have B rows)
 };
-template <int C, int W>
+// G = true: the guided tail (one CTA per guided sample b and band).  It stages two bands, rows b and b + B of img_pre,
+// one after the other so that the staging needs the registers of one band; shared memory doubles (C = 4, W = 64:
+// 43008 B per CTA by -Xptxas -v, so 4 CTAs still fit an SM).  G = false compiles to the same SASS as before.
+template <int C, int W, bool G = false>
 __global__ void __launch_bounds__(256, 4) step_tail_kernel(const __grid_constant__ TailArgs a) {
     constexpr int SW = W + 8, SH = CONV_BAND + 2, w4 = W / 4;
-    constexpr int N_STAGE = C * SH * (w4 + 2);          // float4 slots of the staged band (halo columns included)
     constexpr int N_ITEMS = C * CONV_BAND * w4;          // (output channel, row, 4-pixel group) work items
-    __shared__ __align__(16) float conv_smem[C * SH * SW];
+    constexpr int BAND = C * SH * SW;                    // floats of one staged band
+    __shared__ __align__(16) float conv_smem[(G ? 2 : 1) * BAND];
     __shared__ float sw[C * C * 9 + C];
     const int H = a.H;
     const int bands = H / CONV_BAND;
@@ -531,8 +539,13 @@ __global__ void __launch_bounds__(256, 4) step_tail_kernel(const __grid_constant
     const int t_next = a.next_t[t], late_next = a.next_t[1000 + t];
     const float4 kc = *reinterpret_cast<const float4*>(a.coef + t * 4);
     const unsigned long long seed = ld_state(a.seed_dev), off4 = ld_state(a.seed_dev + 1);
-    // band of the decoder image: all loads of a thread are in flight before its first shared-memory store
-    {
+    // band of the decoder image (guided: row b, then row b + B): all loads of a thread are in flight before its first
+    // shared-memory store
+#pragma unroll 1
+    for (int h = 0; h < (G ? 2 : 1); ++h) {
+        const int src = h ? b + a.B : b;
+        float* band = conv_smem + h * BAND;
+        constexpr int N_STAGE = C * SH * (w4 + 2);  // float4 slots of the staged band (halo columns included)
         constexpr int PER = (N_STAGE + 255) / 256;
         float4 v[PER];
 #pragma unroll
@@ -542,13 +555,13 @@ __global__ void __launch_bounds__(256, 4) step_tail_kernel(const __grid_constant
             const int yy = y0 - 1 + r;
             v[j] = make_float4(0.f, 0.f, 0.f, 0.f);
             if (i < N_STAGE && q >= 1 && q <= w4 && yy >= 0 && yy < H)
-                v[j] = __ldg(reinterpret_cast<const float4*>(a.img_pre + (((size_t)b * C + c) * H + yy) * W) + (q - 1));
+                v[j] = __ldg(reinterpret_cast<const float4*>(a.img_pre + (((size_t)src * C + c) * H + yy) * W) + (q - 1));
         }
 #pragma unroll
         for (int j = 0; j < PER; ++j) {
             const int i = threadIdx.x + j * 256;
             const int q = i % (w4 + 2), r = (i / (w4 + 2)) % SH, c = i / ((w4 + 2) * SH);
-            if (i < N_STAGE) *reinterpret_cast<float4*>(conv_smem + (c * SH + r) * SW + q * 4) = v[j];
+            if (i < N_STAGE) *reinterpret_cast<float4*>(band + (c * SH + r) * SW + q * 4) = v[j];
         }
     }
     const StepCoef k{kc.x, kc.y, kc.z, kc.w};
@@ -565,6 +578,14 @@ __global__ void __launch_bounds__(256, 4) step_tail_kernel(const __grid_constant
         if (t > 0 && a.z_all) zv = reinterpret_cast<const float4*>(a.z_all + (size_t)t * a.n)[e4];
         float acc[4];
         conv_pixels4_one<C>(conv_smem, sw, co, yy, xq, W, acc);
+        if constexpr (G) {
+            // eps = c + s * (c - u), each operation rounded on its own (no FMA contraction): three torch ops give
+            // the same bits
+            float u[4];
+            conv_pixels4_one<C>(conv_smem + BAND, sw, co, yy, xq, W, u);
+#pragma unroll
+            for (int p = 0; p < 4; ++p) acc[p] = __fadd_rn(acc[p], __fmul_rn(a.scale, __fsub_rn(acc[p], u[p])));
+        }
         const float4 ev = make_float4(acc[0], acc[1], acc[2], acc[3]);
         if (t > 0 && !a.z_all) zv = philox_normal4(e4 + off4, t, seed);
         const float4 o = ddpm_update4(a.mode, k, xv, ev, zv);
@@ -574,11 +595,20 @@ __global__ void __launch_bounds__(256, 4) step_tail_kernel(const __grid_constant
         // head of the next step: the updated pixels as bf16 hi | lo patch-vector entries (P = 2: two patches)
         patch_store_pair(patch_elem(tg.a_patch, b, co, y0 + yy, 4 * xq, P, Hp, Wp), o.x, o.y);
         patch_store_pair(patch_elem(tg.a_patch, b, co, y0 + yy, 4 * xq + 2, P, Hp, Wp), o.z, o.w);
+        if constexpr (G) {  // the unconditional row sees the same x
+            patch_store_pair(patch_elem(tg.a_patch, b + a.B, co, y0 + yy, 4 * xq, P, Hp, Wp), o.x, o.y);
+            patch_store_pair(patch_elem(tg.a_patch, b + a.B, co, y0 + yy, 4 * xq + 2, P, Hp, Wp), o.z, o.w);
+        }
     }
-    if (y0 == 0)  // one CTA per sample also writes the next step's time / label token rows
+    if (y0 == 0) {  // one CTA per sample also writes the next step's time / label token rows
         write_token_extras(b, (float)t_next, a.y, tg.pos, tg.label_emb, tg.tokens, tg.stats_p, tg.D, tg.L, tg.extras,
                            tg.normalize_t, tg.num_classes,
                            tg.time_tab ? tg.time_tab + (size_t)min(max(t_next, 0), 999) * tg.D : nullptr);
+        if constexpr (G)  // row b + B: a.y holds [y ; null label] (2B entries)
+            write_token_extras(b + a.B, (float)t_next, a.y, tg.pos, tg.label_emb, tg.tokens, tg.stats_p, tg.D, tg.L,
+                               tg.extras, tg.normalize_t, tg.num_classes,
+                               tg.time_tab ? tg.time_tab + (size_t)min(max(t_next, 0), 999) * tg.D : nullptr);
+    }
     // every CTA has read t above; the last one to get here advances the step counter
     __syncthreads();
     if (threadIdx.x == 0) {

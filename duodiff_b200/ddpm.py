@@ -95,16 +95,21 @@ _SAMPLER_CACHE: "dict[tuple, Sampler]" = {}
 
 
 def cached_sampler(early: Engine, late: "Engine | None", t_switch, batch: int, rule: str = "predict_noise",
-                   variance: str = "beta_tilde", ee_threshold: "float | None" = None, ee_mode: int = 0) -> "Sampler":
-    """Sampler for this (models, batch, rule): its buffers and captured CUDA graphs are reused across get_samples()
-    calls (the graphs read t, the seed and x from sampler-owned device memory, so they do not depend on the call)."""
+                   variance: str = "beta_tilde", ee_threshold: "float | None" = None, ee_mode: int = 0,
+                   guidance: "tuple | None" = None) -> "Sampler":
+    """Sampler for this (models, batch, rule, guidance): its buffers and captured CUDA graphs are reused across
+    get_samples() calls (the graphs read t, the seed and x from sampler-owned device memory, so they do not depend on
+    the call)."""
     key = (early.handle.value, late.handle.value if late is not None else None, switch_step(t_switch), batch, rule,
            variance, ee_threshold, ee_mode)
+    if guidance is not None:
+        key += (("guidance", float(guidance[0]), int(guidance[1])),)
     smp = _SAMPLER_CACHE.get(key)
     if smp is None:
         while len(_SAMPLER_CACHE) >= 4:  # bounded: each entry owns a few x-sized device buffers and two graphs
             _SAMPLER_CACHE.pop(next(iter(_SAMPLER_CACHE)))
-        smp = _SAMPLER_CACHE[key] = Sampler(early, late, t_switch, batch, rule, variance, ee_threshold, ee_mode)
+        smp = _SAMPLER_CACHE[key] = Sampler(early, late, t_switch, batch, rule, variance, ee_threshold, ee_mode,
+                                            guidance=guidance)
     return smp
 
 
@@ -112,7 +117,10 @@ class Sampler:
     """get_samples()' inner loop (sampler.py:128-139 / eesampler.py:57-82) as one C call."""
 
     def __init__(self, early: Engine, late: Engine | None, t_switch, batch: int, rule: str = "predict_noise",
-                 variance: str = "beta_tilde", ee_threshold: float | None = None, ee_mode: int = 0):
+                 variance: str = "beta_tilde", ee_threshold: float | None = None, ee_mode: int = 0,
+                 guidance: "tuple | None" = None):
+        """guidance: (scale, null_label) for classifier-free guidance (ddb_sampler_set_guidance): each step runs the
+        backbones on 2 * batch rows, so both engines need max_batch >= 2 * batch; runs then need labels y."""
         self.lib = _lib.load()
         self.early, self.late, self.batch = early, late, batch
         if isinstance(rule, tuple) and rule[0] == "ddim":  # ("ddim", ddim_steps, ddim_eta)
@@ -133,6 +141,9 @@ class Sampler:
                 0.0 if ee_threshold is None else float(ee_threshold), -1 if ee_threshold is None else int(ee_mode),
                 C.byref(handle)))
         self.handle = handle
+        if guidance is not None:
+            with torch.cuda.device(self.device):
+                _lib.check(self.lib.ddb_sampler_set_guidance(handle, float(guidance[0]), int(guidance[1])))
 
     def __del__(self):
         h = getattr(self, "handle", None)

@@ -9,8 +9,9 @@ update — runs inside libduodiff_b200.so as CUDA-graph replays of hand-written 
 from __future__ import annotations
 
 import functools
+import math
 import time
-from argparse import ArgumentParser
+from argparse import SUPPRESS, ArgumentParser
 from pathlib import Path
 from typing import List
 
@@ -77,10 +78,33 @@ def _ddim_plan(ddim_steps: int, late_available: bool, t_switch):
     return steps, flags
 
 
+def _guidance(models, y, cfg_scale, null_label):
+    """(scale, null_label) of classifier-free guidance, checked against every backbone of the run."""
+    from .early_exit import EarlyExitUViT
+    if y is None:
+        raise ValueError("cfg_scale needs class labels y: guidance contrasts y with the null label")
+    for m in models:
+        if isinstance(m, EarlyExitUViT):
+            raise ValueError("cfg_scale is not supported with early exit: the conditional and unconditional rows "
+                             "would leave at different layers")
+        if getattr(m, "num_classes", 0) <= 0:
+            raise ValueError("cfg_scale needs a class-conditional model (num_classes > 0)")
+    scale = float(cfg_scale)
+    if not math.isfinite(scale):
+        raise ValueError(f"cfg_scale must be finite, got {cfg_scale!r}")
+    # U-ViT's convention: the last row of the label table is the null ("unconditional") label
+    null = models[0].num_classes - 1 if null_label is None else int(null_label)
+    for m in models:
+        if not 0 <= null < m.num_classes:
+            raise ValueError(f"null_label {null} is outside [0, {m.num_classes})")
+    return scale, null
+
+
 def get_samples(model, batch_size: int, postprocessing, seed: int, num_channels: int, sample_height: int,
                 sample_width: int, use_ddim: bool = False, ddim_steps: int = 50, ddim_eta: float = 0.0,
                 timesteps_save: List[int] = (), y=None, autoencoder=None, late_model=None, t_switch=np.inf, *,
-                noise=None, use_graph: bool = True, device=None, x_T=None, noise_row_offset: int = 0):
+                noise=None, use_graph: bool = True, device=None, x_T=None, noise_row_offset: int = 0,
+                cfg_scale=None, null_label=None):
     """sampler.py:82-155.  Returns (samples [B,H,W,C] f32 numpy un-clipped, [intermediate samples]).
 
     x_T is drawn on the CPU generator after ``seed_everything(seed)`` exactly like the reference (sampler.py:99-100);
@@ -92,7 +116,15 @@ def get_samples(model, batch_size: int, postprocessing, seed: int, num_channels:
 
     Sharded (data-parallel) use, see duodiff_b200.distributed: ``x_T`` [B,C,H,W] replaces the draw of the initial
     noise (this rank's rows of the global draw) and ``noise_row_offset`` is the global index of its first row, which
-    keys the Philox stream -- the shards of a global batch then reproduce the single-process result row for row."""
+    keys the Philox stream -- the shards of a global batch then reproduce the single-process result row for row.
+
+    Classifier-free guidance (not in the reference): with ``cfg_scale`` s every step runs the backbone on 2B rows,
+    labels ``y`` and ``null_label`` (default num_classes - 1, U-ViT's null row), and uses eps = eps_c + s * (eps_c -
+    eps_u); s = 0 gives the unguided samples.  It helps only checkpoints trained with label dropout to that row.
+    ``cfg_scale=None`` runs the unguided path unchanged."""
+    guidance = None
+    if cfg_scale is not None:
+        guidance = _guidance([m for m in (model, late_model) if m is not None], y, cfg_scale, null_label)
     dev = _pick_device(model, device)
     _io.seed_everything(seed)
     if x_T is None:
@@ -104,8 +136,9 @@ def get_samples(model, batch_size: int, postprocessing, seed: int, num_channels:
                              f"{(batch_size, num_channels, sample_height, sample_width)}")
     x = x.pin_memory().to(dev, non_blocking=True)
     with torch.cuda.device(dev):
-        early = model.engine(batch_size)
-        late = late_model.engine(batch_size) if late_model is not None else None
+        rows = batch_size if guidance is None else 2 * batch_size  # guided forwards run on [x ; x]
+        early = model.engine(rows)
+        late = late_model.engine(rows) if late_model is not None else None
         if noise is not None:
             noise = noise.to(device=dev, dtype=torch.float32).contiguous()
         # reference: `if 1000 - t in timesteps_save` after the update at t -> save x after the step at t = 1000 - s
@@ -118,7 +151,8 @@ def get_samples(model, batch_size: int, postprocessing, seed: int, num_channels:
                 lat = autoencoder.decode(lat).contiguous()
             return sampler.finalize(lat)
         if use_ddim:
-            sampler = cached_sampler(early, late, t_switch, batch_size, rule=("ddim", int(ddim_steps), float(ddim_eta)))
+            sampler = cached_sampler(early, late, t_switch, batch_size, rule=("ddim", int(ddim_steps), float(ddim_eta)),
+                                     guidance=guidance)
             sampler.set_noise_offset(noise_row_offset)
             steps, flags = _ddim_plan(int(ddim_steps), late is not None, t_switch)
             k0 = 0
@@ -130,7 +164,8 @@ def get_samples(model, batch_size: int, postprocessing, seed: int, num_channels:
                         kept.append(finalize(x))
                     k0 = k + 1
         else:
-            sampler = cached_sampler(early, late, t_switch, batch_size, rule=_rule_name(postprocessing))
+            sampler = cached_sampler(early, late, t_switch, batch_size, rule=_rule_name(postprocessing),
+                                     guidance=guidance)
             sampler.set_noise_offset(noise_row_offset)
             t_first = 999
             for t_stop in sorted((t for t in save_at if 0 <= t <= 999), reverse=True) + [0]:
@@ -178,7 +213,14 @@ def get_args(argv=None):
     p.add_argument("--ddim_steps", type=int, default=50)
     p.add_argument("--ddim_eta", type=float, default=0.0)
     p.add_argument("--timesteps_save", type=int, nargs="+", default=[])
-    return p.parse_args(argv)
+    # not a flag of the reference: absent from the namespace unless given, so unguided runs parse exactly as before
+    p.add_argument("--cfg_scale", type=float, default=SUPPRESS,
+                   help="Classifier-free guidance scale s: eps = eps_c + s * (eps_c - eps_u) against the null label "
+                        "num_classes - 1 (needs --class_id)")
+    args = p.parse_args(argv)
+    if getattr(args, "cfg_scale", None) is not None and args.class_id is None:
+        p.error("--cfg_scale needs --class_id: guidance contrasts the class labels with the null label")
+    return args
 
 
 def draw_labels(batch_size: int, num_classes: int):
@@ -201,6 +243,7 @@ def main(argv=None):
     """The reference's CLI.  Under `torchrun --nproc-per-node N` each rank samples its shard of the --batch_size
     images (duodiff_b200.distributed) and rank 0 writes exactly the files a single process writes."""
     args = get_args(argv)
+    cfg_scale = getattr(args, "cfg_scale", None)
     out_dir = Path(args.output_folder)
     if D.env_rank_world()[0] == 0:
         out_dir.mkdir(parents=True, exist_ok=True)
@@ -210,10 +253,11 @@ def main(argv=None):
         print(f"Using device {device}")
         lo, hi = D.shard_bounds(args.batch_size, rank, world)
         model = late = autoencoder = None
+        rows = (hi - lo) * (2 if cfg_scale is not None else 1)  # a guided forward runs on 2B rows
         if hi > lo:  # a rank with an empty shard (more ranks than images) builds nothing
-            model, cfg = _build(args.config_path, args.checkpoint_path, hi - lo, device)
+            model, cfg = _build(args.config_path, args.checkpoint_path, rows, device)
             if args.checkpoint_path_late:
-                late, cfg = _build(args.config_path_late, args.checkpoint_path_late, hi - lo, device)
+                late, cfg = _build(args.config_path_late, args.checkpoint_path_late, rows, device)
         else:
             cfg = _io.load_config(args.config_path_late if args.checkpoint_path_late else args.config_path)
         mp = cfg["model_params"]
@@ -221,6 +265,12 @@ def main(argv=None):
         y = None
         if args.class_id is not None:
             y = draw_labels(args.batch_size, mp.get("num_classes", -1)).to(device)
+        guided = {}
+        if cfg_scale is not None:
+            guided = dict(cfg_scale=cfg_scale, null_label=mp.get("num_classes", -1) - 1)
+            if rank == 0:
+                print(f"Classifier-free guidance: scale {cfg_scale}, null label {guided['null_label']} "
+                      f"(the last row of the {mp.get('num_classes', -1)}-row label table)")
         if "autoencoder" in cfg and hi > lo:  # sampler.py:320-325
             autoencoder = get_autoencoder(cfg["autoencoder"]["autoencoder_checkpoint_path"])
         D.barrier()  # every rank has loaded its models: the clock starts together
@@ -231,7 +281,7 @@ def main(argv=None):
             postprocessing=_BY_NAME[args.parametrization], num_channels=mp["in_chans"],
             sample_height=mp["img_size"], sample_width=mp["img_size"], use_ddim=args.use_ddim,
             ddim_steps=args.ddim_steps, ddim_eta=args.ddim_eta, autoencoder=autoencoder, late_model=late,
-            t_switch=args.t_switch, timesteps_save=args.timesteps_save)
+            t_switch=args.t_switch, timesteps_save=args.timesteps_save, **guided)
         D.barrier()  # every shard is done: what follows is the gather alone
         t_gather = time.time()
         result = D.gather_to_rank0(local, args.batch_size, D.SAMPLER_OUTPUTS)

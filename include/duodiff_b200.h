@@ -117,6 +117,13 @@ int ddb_ddpm_step(float* x_dev, const float* model_out_dev, const float* z_dev, 
 int ddb_sampler_create(ddb_model* early, ddb_model* late, int32_t switch_t, int32_t B, const float* coef_host,
                        int32_t step_mode, float ee_threshold, int32_t ee_mode, ddb_sampler** out);
 void ddb_sampler_destroy(ddb_sampler* s);
+/* Classifier-free guidance (U-ViT's form): every step runs the backbone on 2B rows, the conditional half with the
+ * caller's labels y and the unconditional half with `null_label`, and the step tail uses
+ * eps = eps_c + scale * (eps_c - eps_u) (scale 0 gives eps_c) per sample.  x, the noise keying and the traces stay
+ * per sample (B rows).  Call once before the first run.  Fails with DDB_ERR_INVALID when a backbone is unconditional,
+ * null_label is outside [0, num_classes) of a backbone, a backbone's max_batch < 2B, the scale is not finite, or the
+ * sampler has early exit (ee_mode >= 0). */
+int ddb_sampler_set_guidance(ddb_sampler* s, float scale, int64_t null_label);
 /* Data-parallel sharding: `first_row` = index of this shard's first sample in the global batch (default 0).  The
  * in-kernel Philox noise is keyed by (seed, t, GLOBAL element index), so the shards of a global batch draw exactly the
  * z_t a single-GPU run of the whole batch draws: N-GPU sampling == 1-GPU sampling row for row (SURVEY.md 8e). */
