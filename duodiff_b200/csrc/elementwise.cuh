@@ -436,6 +436,22 @@ __device__ __forceinline__ float4 ddpm_update4(int mode, const StepCoef& k, floa
     return make_float4(ddpm_update1(mode, k, x.x, e.x, z.x), ddpm_update1(mode, k, x.y, e.y, z.y),
                        ddpm_update1(mode, k, x.z, e.z, z.z), ddpm_update1(mode, k, x.w, e.w, z.w));
 }
+// DPM-Solver++(2M), mode 3 (ddpm.dpm_solver_coefficients): row {a, b, rho, phi | w0, w1, order, 0}.  No noise term.
+//   D_t = a*x + b*out;  D = w0*D_t + w1*D_prev (order 2) or D_t (order 1);  x' = rho*x + phi*D;  D_prev <- D_t
+// Every operation rounded on its own (no FMA contraction), so torch elementwise ops give the same bits.  An order-1
+// step never reads D_prev: a stale or uninitialised buffer cannot reach x.
+struct MsCoef {
+    float a, b, rho, phi, w0, w1;
+};
+__device__ __forceinline__ float ms_update1(const MsCoef& k, bool second, float x, float e, float dp, float& dt) {
+    dt = __fadd_rn(__fmul_rn(k.a, x), __fmul_rn(k.b, e));
+    const float d = second ? __fadd_rn(__fmul_rn(k.w0, dt), __fmul_rn(k.w1, dp)) : dt;
+    return __fadd_rn(__fmul_rn(k.rho, x), __fmul_rn(k.phi, d));
+}
+__device__ __forceinline__ float4 ms_update4(const MsCoef& k, bool second, float4 x, float4 e, float4 dp, float4& dt) {
+    return make_float4(ms_update1(k, second, x.x, e.x, dp.x, dt.x), ms_update1(k, second, x.y, e.y, dp.y, dt.y),
+                       ms_update1(k, second, x.z, e.z, dp.z, dt.z), ms_update1(k, second, x.w, e.w, dp.w, dt.w));
+}
 
 // seed_dev (graph replay / sampler): {Philox key, float4 index of this shard's first element in the global batch}
 __global__ void __launch_bounds__(256) ddpm_step_kernel(float* __restrict__ x, const float* __restrict__ model_out,
@@ -486,7 +502,7 @@ struct TailArgs {
     const float* conv_b;
     float* x;              // [B,C,H,W] in place
     const float* z_all;    // injected noise [1000, n] or null (Philox)
-    const float* coef;     // [1000,4]
+    const float* coef;     // [1000,4]; mode 3 (DPM-Solver++): [1000,8]
     int* t_dev;            // step counter (read by every CTA, advanced by the last one to finish)
     const int* next_t;     // [1000] successor table; [1000, 2000): 1 = the step after t runs on the late backbone
     const unsigned long long* seed_dev;  // {Philox key, float4 offset of the shard in the global batch}
@@ -509,11 +525,16 @@ struct TailArgs {
     int guide;             // 0 / 1; selects the G = true instantiation on the host
     float scale;
     int B;                 // guided samples (x, noise and traces have B rows)
+    // DPM-Solver++(2M) (mode 3, MS = true): the previous step's data prediction D_prev [B,C,H,W], sampler-owned
+    float* d_prev;
 };
 // G = true: the guided tail (one CTA per guided sample b and band).  It stages two bands, rows b and b + B of img_pre,
 // one after the other so that the staging needs the registers of one band; shared memory doubles (C = 4, W = 64:
 // 43008 B per CTA by -Xptxas -v, so 4 CTAs still fit an SM).  G = false compiles to the same SASS as before.
-template <int C, int W, bool G = false>
+// MS = true: the multistep update of mode 3 (ms_update4) replaces the DDPM / DDIM one; it reads the 8-float row as two
+// float4 and D_prev (order-2 rows only) at the element the thread owns, and writes D_t there.  MS = false compiles to
+// the same SASS as before.
+template <int C, int W, bool G = false, bool MS = false>
 __global__ void __launch_bounds__(256, 4) step_tail_kernel(const __grid_constant__ TailArgs a) {
     constexpr int SW = W + 8, SH = CONV_BAND + 2, w4 = W / 4;
     constexpr int N_ITEMS = C * CONV_BAND * w4;          // (output channel, row, 4-pixel group) work items
@@ -537,7 +558,9 @@ __global__ void __launch_bounds__(256, 4) step_tail_kernel(const __grid_constant
     const int t = ld_state(a.t_dev);
     // everything that depends on t is requested at once (one further round trip, not three)
     const int t_next = a.next_t[t], late_next = a.next_t[1000 + t];
-    const float4 kc = *reinterpret_cast<const float4*>(a.coef + t * 4);
+    const float4 kc = *reinterpret_cast<const float4*>(a.coef + t * (MS ? 8 : 4));
+    float4 kc2;
+    if constexpr (MS) kc2 = *reinterpret_cast<const float4*>(a.coef + t * 8 + 4);
     const unsigned long long seed = ld_state(a.seed_dev), off4 = ld_state(a.seed_dev + 1);
     // band of the decoder image (guided: row b, then row b + B): all loads of a thread are in flight before its first
     // shared-memory store
@@ -574,8 +597,12 @@ __global__ void __launch_bounds__(256, 4) step_tail_kernel(const __grid_constant
         const size_t e4 = ((((size_t)b * C + co) * H + y0 + yy) * W) / 4 + xq;  // float4 index inside the shard
         // x (and the injected noise) do not depend on the conv: their loads are in flight while it is computed
         const float4 xv = reinterpret_cast<const float4*>(a.x)[e4];
-        float4 zv = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (t > 0 && a.z_all) zv = reinterpret_cast<const float4*>(a.z_all + (size_t)t * a.n)[e4];
+        float4 zv = make_float4(0.f, 0.f, 0.f, 0.f);  // MS: D_prev
+        if constexpr (MS) {
+            if (kc2.z == 2.f) zv = reinterpret_cast<const float4*>(a.d_prev)[e4];
+        } else if (t > 0 && a.z_all) {
+            zv = reinterpret_cast<const float4*>(a.z_all + (size_t)t * a.n)[e4];
+        }
         float acc[4];
         conv_pixels4_one<C>(conv_smem, sw, co, yy, xq, W, acc);
         if constexpr (G) {
@@ -587,8 +614,15 @@ __global__ void __launch_bounds__(256, 4) step_tail_kernel(const __grid_constant
             for (int p = 0; p < 4; ++p) acc[p] = __fadd_rn(acc[p], __fmul_rn(a.scale, __fsub_rn(acc[p], u[p])));
         }
         const float4 ev = make_float4(acc[0], acc[1], acc[2], acc[3]);
-        if (t > 0 && !a.z_all) zv = philox_normal4(e4 + off4, t, seed);
-        const float4 o = ddpm_update4(a.mode, k, xv, ev, zv);
+        float4 o;
+        if constexpr (MS) {
+            float4 dt;
+            o = ms_update4(MsCoef{kc.x, kc.y, kc.z, kc.w, kc2.x, kc2.y}, kc2.z == 2.f, xv, ev, zv, dt);
+            reinterpret_cast<float4*>(a.d_prev)[e4] = dt;
+        } else {
+            if (t > 0 && !a.z_all) zv = philox_normal4(e4 + off4, t, seed);
+            o = ddpm_update4(a.mode, k, xv, ev, zv);
+        }
         reinterpret_cast<float4*>(a.x)[e4] = o;
         if (a.eps_out) reinterpret_cast<float4*>(a.eps_out)[e4] = ev;
         if (a.x_save) reinterpret_cast<float4*>(a.x_save)[e4] = o;

@@ -2,6 +2,7 @@
 from __future__ import annotations
 
 import ctypes as C
+import math
 
 import torch
 
@@ -37,6 +38,40 @@ def ddim_coefficients(ddim_steps: int, ddim_eta: float):
         table[t, 2] = sigma2 if s > 0 else 0.0
         table[t, 3] = torch.sqrt(1 - ab[s] - sigma2)
     return table.contiguous(), 2
+
+
+def dpm_solver_coefficients(steps: int, parametrization: str = "predict_noise"):
+    """[1000,8] fp32 table {a, b, rho, phi, w0, w1, order, 0} of DPM-Solver++(2M), mode 3 of the step kernel, over
+    the DDIM grid ddim_timesteps(steps) (steps - 1 model evaluations).  With alpha = sqrt(abar), sigma = sqrt(1 - abar),
+    lambda = log(alpha / sigma), the step from t to the next grid point s, h = lambda_s - lambda_t, r = h_prev / h:
+        D_t = a*x + b*out            predict_noise: a = 1/alpha_t, b = -sigma_t/alpha_t;  predict_original: a = 0, b = 1
+        D   = w0*D_t + w1*D_prev     order 2: w0 = 1 + 1/(2r), w1 = -1/(2r);  order 1: D = D_t (w0 = 1, w1 = 0)
+        x'  = rho*x + phi*D          rho = sigma_s/sigma_t, phi = alpha_s * (-expm1(-h));  D_prev <- D_t
+    The first step is order 1, and so is the final one when the grid has fewer than 15 model evaluations (the usual
+    lower_order_final rule: h of the step to t = 0 is large).  Computed in fp64 from the fp32 schedule, rounded once.
+    Rows of timesteps no step starts from have order 0."""
+    if parametrization not in ("predict_noise", "predict_original"):
+        raise ValueError(f"DPM-Solver++ needs a data or noise prediction, not {parametrization!r}")
+    if int(steps) < 2:
+        raise ValueError(f"dpm_solver_steps={steps}: the grid needs at least 2 points (one model evaluation)")
+    ab = schedule()["alphas_bar"].double()
+    alpha, sigma = ab.sqrt(), (1 - ab).sqrt()
+    lam = alpha.log() - sigma.log()
+    ts = ddim_timesteps(int(steps))
+    evals = len(ts) - 1
+    table = torch.zeros(1000, 8, dtype=torch.float64)
+    for k, (t, s) in enumerate(zip(ts[:-1], ts[1:])):
+        h = float(lam[s] - lam[t])
+        order = 1 if k == 0 or (k == evals - 1 and evals < 15) else 2
+        w0, w1 = 1.0, 0.0
+        if order == 2:
+            r = float(lam[t] - lam[ts[k - 1]]) / h
+            w0, w1 = 1 + 1 / (2 * r), -1 / (2 * r)
+        a, b = (0.0, 1.0) if parametrization == "predict_original" else (float(1 / alpha[t]),
+                                                                        float(-sigma[t] / alpha[t]))
+        table[t] = torch.tensor([a, b, float(sigma[s] / sigma[t]), float(alpha[s]) * -math.expm1(-h), w0, w1, order,
+                                 0.0], dtype=torch.float64)
+    return table.to(torch.float32).contiguous(), 3
 
 
 def schedule() -> dict:
@@ -125,6 +160,8 @@ class Sampler:
         self.early, self.late, self.batch = early, late, batch
         if isinstance(rule, tuple) and rule[0] == "ddim":  # ("ddim", ddim_steps, ddim_eta)
             table, mode = ddim_coefficients(int(rule[1]), float(rule[2]))
+        elif isinstance(rule, tuple) and rule[0] == "dpm_solver++":  # ("dpm_solver++", steps, parametrization)
+            table, mode = dpm_solver_coefficients(int(rule[1]), rule[2])
         else:
             table, mode = step_coefficients(rule, variance)
         self.coef = table

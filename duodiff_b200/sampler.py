@@ -100,11 +100,26 @@ def _guidance(models, y, cfg_scale, null_label):
     return scale, null
 
 
+def _dpm_solver_rule(models, postprocessing, use_ddim, steps):
+    """Sampler rule ("dpm_solver++", steps, parametrization) of DPM-Solver++(2M), checked against the run."""
+    from .early_exit import EarlyExitUViT
+    if use_ddim:
+        raise ValueError("dpm_solver_steps and use_ddim select two different samplers: give one of them")
+    name = _rule_name(postprocessing)
+    if name == "predict_previous":
+        raise ValueError("DPM-Solver++ needs a noise or data prediction, not predict_previous")
+    if int(steps) < 2:
+        raise ValueError(f"dpm_solver_steps={steps}: the grid needs at least 2 points (one model evaluation)")
+    if any(isinstance(m, EarlyExitUViT) for m in models):
+        raise ValueError("dpm_solver_steps is not supported with early exit")
+    return "dpm_solver++", int(steps), name
+
+
 def get_samples(model, batch_size: int, postprocessing, seed: int, num_channels: int, sample_height: int,
                 sample_width: int, use_ddim: bool = False, ddim_steps: int = 50, ddim_eta: float = 0.0,
                 timesteps_save: List[int] = (), y=None, autoencoder=None, late_model=None, t_switch=np.inf, *,
                 noise=None, use_graph: bool = True, device=None, x_T=None, noise_row_offset: int = 0,
-                cfg_scale=None, null_label=None):
+                cfg_scale=None, null_label=None, dpm_solver_steps=None):
     """sampler.py:82-155.  Returns (samples [B,H,W,C] f32 numpy un-clipped, [intermediate samples]).
 
     x_T is drawn on the CPU generator after ``seed_everything(seed)`` exactly like the reference (sampler.py:99-100);
@@ -121,10 +136,19 @@ def get_samples(model, batch_size: int, postprocessing, seed: int, num_channels:
     Classifier-free guidance (not in the reference): with ``cfg_scale`` s every step runs the backbone on 2B rows,
     labels ``y`` and ``null_label`` (default num_classes - 1, U-ViT's null row), and uses eps = eps_c + s * (eps_c -
     eps_u); s = 0 gives the unguided samples.  It helps only checkpoints trained with label dropout to that row.
-    ``cfg_scale=None`` runs the unguided path unchanged."""
+    ``cfg_scale=None`` runs the unguided path unchanged.
+
+    DPM-Solver++(2M) (not in the reference): ``dpm_solver_steps`` n runs the second-order multistep solver of the
+    probability-flow ODE over the DDIM grid (n - 1 model evaluations at the timesteps of ``use_ddim=True,
+    ddim_steps=n``), with the hand-off, ``timesteps_save``, ``autoencoder`` and ``cfg_scale`` as in the DDIM branch.
+    It has no noise term.  ``postprocessing`` must be predict_noise or predict_original."""
+    models = [m for m in (model, late_model) if m is not None]
     guidance = None
     if cfg_scale is not None:
-        guidance = _guidance([m for m in (model, late_model) if m is not None], y, cfg_scale, null_label)
+        guidance = _guidance(models, y, cfg_scale, null_label)
+    dpm_rule = None
+    if dpm_solver_steps is not None:
+        dpm_rule = _dpm_solver_rule(models, postprocessing, use_ddim, dpm_solver_steps)
     dev = _pick_device(model, device)
     _io.seed_everything(seed)
     if x_T is None:
@@ -150,11 +174,12 @@ def get_samples(model, batch_size: int, postprocessing, seed: int, num_channels:
                 print("Decode the images...")
                 lat = autoencoder.decode(lat).contiguous()
             return sampler.finalize(lat)
-        if use_ddim:
-            sampler = cached_sampler(early, late, t_switch, batch_size, rule=("ddim", int(ddim_steps), float(ddim_eta)),
-                                     guidance=guidance)
+        if use_ddim or dpm_rule is not None:
+            # DDIM and DPM-Solver++ walk the same grid; after the step at t in save_at x is saved
+            rule = dpm_rule or ("ddim", int(ddim_steps), float(ddim_eta))
+            sampler = cached_sampler(early, late, t_switch, batch_size, rule=rule, guidance=guidance)
             sampler.set_noise_offset(noise_row_offset)
-            steps, flags = _ddim_plan(int(ddim_steps), late is not None, t_switch)
+            steps, flags = _ddim_plan(rule[1], late is not None, t_switch)
             k0 = 0
             for k, t in enumerate(steps):
                 if t in save_at or k == len(steps) - 1:
@@ -217,9 +242,19 @@ def get_args(argv=None):
     p.add_argument("--cfg_scale", type=float, default=SUPPRESS,
                    help="Classifier-free guidance scale s: eps = eps_c + s * (eps_c - eps_u) against the null label "
                         "num_classes - 1 (needs --class_id)")
+    p.add_argument("--dpm_solver_steps", type=int, default=SUPPRESS,
+                   help="Sample with DPM-Solver++(2M) over the DDIM grid of N points (N - 1 model evaluations, the "
+                        "timesteps of --use_ddim --ddim_steps N); no noise term")
     args = p.parse_args(argv)
     if getattr(args, "cfg_scale", None) is not None and args.class_id is None:
         p.error("--cfg_scale needs --class_id: guidance contrasts the class labels with the null label")
+    if getattr(args, "dpm_solver_steps", None) is not None:
+        if args.use_ddim:
+            p.error("--dpm_solver_steps and --use_ddim select two different samplers: give one of them")
+        if args.parametrization == "predict_previous":
+            p.error("--dpm_solver_steps needs --parametrization predict_noise or predict_original")
+        if args.dpm_solver_steps < 2:
+            p.error("--dpm_solver_steps needs at least 2 grid points (one model evaluation)")
     return args
 
 
@@ -265,12 +300,14 @@ def main(argv=None):
         y = None
         if args.class_id is not None:
             y = draw_labels(args.batch_size, mp.get("num_classes", -1)).to(device)
-        guided = {}
+        extra = {}  # keywords of the samplers that are not in the reference
         if cfg_scale is not None:
-            guided = dict(cfg_scale=cfg_scale, null_label=mp.get("num_classes", -1) - 1)
+            extra = dict(cfg_scale=cfg_scale, null_label=mp.get("num_classes", -1) - 1)
             if rank == 0:
-                print(f"Classifier-free guidance: scale {cfg_scale}, null label {guided['null_label']} "
+                print(f"Classifier-free guidance: scale {cfg_scale}, null label {extra['null_label']} "
                       f"(the last row of the {mp.get('num_classes', -1)}-row label table)")
+        if getattr(args, "dpm_solver_steps", None) is not None:
+            extra["dpm_solver_steps"] = args.dpm_solver_steps
         if "autoencoder" in cfg and hi > lo:  # sampler.py:320-325
             autoencoder = get_autoencoder(cfg["autoencoder"]["autoencoder_checkpoint_path"])
         D.barrier()  # every rank has loaded its models: the clock starts together
@@ -281,7 +318,7 @@ def main(argv=None):
             postprocessing=_BY_NAME[args.parametrization], num_channels=mp["in_chans"],
             sample_height=mp["img_size"], sample_width=mp["img_size"], use_ddim=args.use_ddim,
             ddim_steps=args.ddim_steps, ddim_eta=args.ddim_eta, autoencoder=autoencoder, late_model=late,
-            t_switch=args.t_switch, timesteps_save=args.timesteps_save, **guided)
+            t_switch=args.t_switch, timesteps_save=args.timesteps_save, **extra)
         D.barrier()  # every shard is done: what follows is the gather alone
         t_gather = time.time()
         result = D.gather_to_rank0(local, args.batch_size, D.SAMPLER_OUTPUTS)
