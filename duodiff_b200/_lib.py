@@ -54,6 +54,8 @@ _SIGS = {
     "ddb_sampler_profile_step": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P]),
     "ddb_sampler_run": (C.c_int, [_P, _P, _P, _P, C.c_uint64, C.c_int32, C.c_int32, _P, _P, _P, _P, C.c_int32, _P]),
     "ddb_sampler_run_list": (C.c_int, [_P, _P, _P, _P, C.c_uint64, _P, _P, C.c_int32, _P, _P, C.c_int32, _P]),
+    "ddb_sampler_run_list_logs": (C.c_int, [_P, _P, _P, _P, C.c_uint64, _P, _P, C.c_int32, _P, _P, _P, _P, C.c_int32,
+                                            _P]),
     "ddb_finalize_nhwc": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P]),
     "ddb_op_gemm": (C.c_int, [_P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, C.c_int32, C.c_int32,
                               C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P]),

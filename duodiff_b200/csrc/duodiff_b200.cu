@@ -1813,11 +1813,11 @@ int ddb_sampler_set_noise_offset(ddb_sampler* s, uint64_t first_row) {
 }
 
 // Runs the model at the timesteps t_list[0..n) (late[k] != 0: on the late backbone) with the sampler's update rule.
-// log_lo..log_hi: rows (timesteps) of the early-exit logs copied to the caller's buffers afterwards.
+// The early-exit log rows of the visited timesteps are copied to the caller's buffers afterwards (when given).
 static int sampler_run_impl(ddb_sampler* s, float* x_dev, const int64_t* y_dev, const float* z_all_dev, uint64_t seed,
                             const int32_t* t_list, const uint8_t* late, int n, float* eps_trace_dev, float* x_trace_dev,
-                            int32_t* exit_idx_trace_dev, float* score_mean_trace_dev, int log_lo, int log_hi,
-                            int32_t use_graph, cudaStream_t st) {
+                            int32_t* exit_idx_trace_dev, float* score_mean_trace_dev, int32_t use_graph,
+                            cudaStream_t st) {
     if (n <= 0) return DDB_OK;
     for (int k = 0; k < n; ++k) {
         if (t_list[k] < 0 || t_list[k] > 999) return fail(DDB_ERR_INVALID, "timestep %d outside [0, 999]", t_list[k]);
@@ -1917,16 +1917,22 @@ static int sampler_run_impl(ddb_sampler* s, float* x_dev, const int64_t* y_dev, 
         }
         CUDA_TRY(cudaMemcpyAsync(x_dev, xw, s->n * 4, cudaMemcpyDeviceToDevice, st));
     }
-    // early-exit logs: the rows of the timesteps this call covered, from the sampler-owned buffers
-    if (log_hi >= log_lo) {
-        const size_t rows = (size_t)(log_hi - log_lo + 1);
-        if (exit_idx_trace_dev)
-            CUDA_TRY(cudaMemcpyAsync(exit_idx_trace_dev + (size_t)log_lo * s->B, s->exit_log->as<int32_t>() + (size_t)log_lo * s->B,
-                                     rows * s->B * 4, cudaMemcpyDeviceToDevice, st));
+    // early-exit logs: the rows of the timesteps this call visited, from the sampler-owned buffers; a run of
+    // consecutive timesteps (t, t-1, ...) is one copy, so a DDPM range is a single copy per log
+    if (exit_idx_trace_dev || score_mean_trace_dev) {
         const int depth = s->early->cfg.depth;
-        if (score_mean_trace_dev)
-            CUDA_TRY(cudaMemcpyAsync(score_mean_trace_dev + (size_t)log_lo * depth, s->score_log->as<float>() + (size_t)log_lo * depth,
-                                     rows * depth * 4, cudaMemcpyDeviceToDevice, st));
+        for (int k = 0; k < n;) {
+            int j = k;
+            while (j + 1 < n && t_list[j + 1] == t_list[j] - 1) ++j;
+            const size_t lo = (size_t)t_list[j], rows = (size_t)(j - k + 1);
+            if (exit_idx_trace_dev)
+                CUDA_TRY(cudaMemcpyAsync(exit_idx_trace_dev + lo * s->B, s->exit_log->as<int32_t>() + lo * s->B,
+                                         rows * s->B * 4, cudaMemcpyDeviceToDevice, st));
+            if (score_mean_trace_dev)
+                CUDA_TRY(cudaMemcpyAsync(score_mean_trace_dev + lo * depth, s->score_log->as<float>() + lo * depth,
+                                         rows * depth * 4, cudaMemcpyDeviceToDevice, st));
+            k = j + 1;
+        }
     }
     return DDB_OK;
 }
@@ -1945,8 +1951,7 @@ int ddb_sampler_run(ddb_sampler* s, float* x_dev, const int64_t* y_dev, const fl
         late.push_back((s->late && t < s->switch_t) ? 1 : 0);  // sampler.py:135-136
     }
     return sampler_run_impl(s, x_dev, y_dev, z_all_dev, seed, ts.data(), late.data(), (int)ts.size(), eps_trace_dev,
-                            x_trace_dev, exit_idx_trace_dev, score_mean_trace_dev, t_last, t_first, use_graph,
-                            (cudaStream_t)stream);
+                            x_trace_dev, exit_idx_trace_dev, score_mean_trace_dev, use_graph, (cudaStream_t)stream);
 }
 
 int ddb_sampler_run_list(ddb_sampler* s, float* x_dev, const int64_t* y_dev, const float* z_all_dev, uint64_t seed,
@@ -1954,7 +1959,16 @@ int ddb_sampler_run_list(ddb_sampler* s, float* x_dev, const int64_t* y_dev, con
                          float* x_trace_dev, int32_t use_graph, void* stream) {
     if (!s || !x_dev || !t_list_host || !late_host) return fail(DDB_ERR_INVALID, "null argument");
     return sampler_run_impl(s, x_dev, y_dev, z_all_dev, seed, t_list_host, late_host, n_steps, eps_trace_dev,
-                            x_trace_dev, nullptr, nullptr, 0, -1, use_graph, (cudaStream_t)stream);
+                            x_trace_dev, nullptr, nullptr, use_graph, (cudaStream_t)stream);
+}
+
+int ddb_sampler_run_list_logs(ddb_sampler* s, float* x_dev, const int64_t* y_dev, const float* z_all_dev,
+                              uint64_t seed, const int32_t* t_list_host, const uint8_t* late_host, int32_t n_steps,
+                              float* eps_trace_dev, float* x_trace_dev, int32_t* exit_idx_trace_dev,
+                              float* score_mean_trace_dev, int32_t use_graph, void* stream) {
+    if (!s || !x_dev || !t_list_host || !late_host) return fail(DDB_ERR_INVALID, "null argument");
+    return sampler_run_impl(s, x_dev, y_dev, z_all_dev, seed, t_list_host, late_host, n_steps, eps_trace_dev,
+                            x_trace_dev, exit_idx_trace_dev, score_mean_trace_dev, use_graph, (cudaStream_t)stream);
 }
 
 int ddb_sampler_profile_step(ddb_sampler* s, float* x_dev, const int64_t* y_dev, int32_t t, int32_t late,
@@ -1965,7 +1979,7 @@ int ddb_sampler_profile_step(ddb_sampler* s, float* x_dev, const int64_t* y_dev,
     const uint8_t lf[1] = {(uint8_t)(late ? 1 : 0)};
     g_prof.active = true, g_prof.st = st, g_prof.used = 0;
     g_prof.cats.clear();
-    int r = sampler_run_impl(s, x_dev, y_dev, nullptr, 0, tl, lf, 1, nullptr, nullptr, nullptr, nullptr, 0, -1, 0, st);
+    int r = sampler_run_impl(s, x_dev, y_dev, nullptr, 0, tl, lf, 1, nullptr, nullptr, nullptr, nullptr, 0, st);
     g_prof.active = false;
     if (r != DDB_OK) return r;
     CUDA_TRY(cudaStreamSynchronize(st));

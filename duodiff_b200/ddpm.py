@@ -233,19 +233,27 @@ class Sampler:
         return x
 
     def run_list(self, x, t_list, late_flags, y=None, noise=None, seed: int = 0, eps_trace=None, x_trace=None,
-                 use_graph: bool = True):
+                 exit_log=None, score_log=None, use_graph: bool = True):
         """The same loop over an explicit timestep list (DDIM): model at t_list[k] (late backbone if late_flags[k]),
-        then the sampler's update with the coefficients of t_list[k]."""
+        then the sampler's update with the coefficients of t_list[k].  exit_log / score_log as in run(): only the rows
+        of the timesteps in t_list are written."""
         y = self._check_xy(x, y, noise)
         n = len(t_list)
         assert n == len(late_flags)
         ts = (C.c_int32 * n)(*[int(t) for t in t_list])
         lf = (C.c_uint8 * n)(*[1 if f else 0 for f in late_flags])
+        for log, dtype, cols in ((exit_log, torch.int32, self.batch), (score_log, torch.float32, self.early.depth)):
+            if log is not None:
+                assert log.is_cuda and log.dtype == dtype and log.is_contiguous() and tuple(log.shape) == (1000, cols)
         graph = bool(use_graph) and eps_trace is None and x_trace is None
+        args = (self.handle, x.data_ptr(), _lib.ptr(y), _lib.ptr(noise), int(seed) & (2**64 - 1), ts, lf, n,
+                _lib.ptr(eps_trace), _lib.ptr(x_trace))
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.ddb_sampler_run_list(
-                self.handle, x.data_ptr(), _lib.ptr(y), _lib.ptr(noise), int(seed) & (2**64 - 1), ts, lf, n,
-                _lib.ptr(eps_trace), _lib.ptr(x_trace), int(graph), _lib.current_stream_ptr()))
+            if exit_log is None and score_log is None:
+                _lib.check(self.lib.ddb_sampler_run_list(*args, int(graph), _lib.current_stream_ptr()))
+            else:
+                _lib.check(self.lib.ddb_sampler_run_list_logs(*args, _lib.ptr(exit_log), _lib.ptr(score_log),
+                                                              int(graph), _lib.current_stream_ptr()))
         return x
 
     def finalize(self, x):

@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import functools
 import time
-from argparse import ArgumentParser
+from argparse import SUPPRESS, ArgumentParser
 from pathlib import Path
 
 import numpy as np
@@ -18,14 +18,15 @@ from . import _io
 from . import distributed as D
 from .autoencoder import get_autoencoder
 from .ddpm import cached_sampler
-from .sampler import _pick_device, draw_labels
+from .sampler import _ddim_plan, _pick_device, draw_labels
 from .early_exit import EarlyExitUViT
 from .uvit import UViT
 
 
 def get_samples(model, batch_size: int, seed: int, num_channels: int, sample_height: int, sample_width: int,
                 threshold: float, depth: int, y=None, autoencoder=None, *, noise=None, mode: int = 0,
-                use_graph: bool = True, device=None, x_T=None, noise_row_offset: int = 0):
+                use_graph: bool = True, device=None, x_T=None, noise_row_offset: int = 0, use_ddim: bool = False,
+                ddim_steps=None, ddim_eta=None):
     """eesampler.py:40-89 -> (samples [B,H,W,C] numpy, error_prediction_by_timestep [1000,depth],
     indices_by_timestep [1000,B]) with both logs as CPU float32 tensors indexed by t like the reference's.
 
@@ -34,7 +35,22 @@ def get_samples(model, batch_size: int, seed: int, num_channels: int, sample_hei
     ``error_prediction_by_timestep`` then holds, per layer, the mean probe output over the samples STILL IN THE BATCH at
     that layer (NaN once the batch is empty) -- the reference's mean over the whole batch (eesampler.py:71) would need
     the skipped layers.  Any ``threshold`` is legal; a negative one selects layer 0's head for every sample, as the
-    reference's argmax over an all-false mask does.  ``x_T`` / ``noise_row_offset``: see sampler.get_samples."""
+    reference's argmax over an all-false mask does.  ``x_T`` / ``noise_row_offset``: see sampler.get_samples.
+
+    DDIM (not in the reference's eesampler.py): ``use_ddim`` walks the strided grid of ``sampler.get_samples(use_ddim=
+    True)`` -- ``ddim_steps`` points (default 50), ``ddim_steps - 1`` model evaluations, the update of sampler.py:110-120
+    with its sigma_t^2 * z noise term scaled by ``ddim_eta`` (default 0) -- with the same early exit at every step.  The
+    logs keep their shapes and dtypes; rows of timesteps the grid does not visit are NaN in both (a row of zeros would
+    read as "every sample left at layer 0").  ``ddim_steps`` / ``ddim_eta`` without ``use_ddim`` raise ValueError."""
+    steps = flags = None
+    if use_ddim:
+        ddim_steps = 50 if ddim_steps is None else int(ddim_steps)
+        ddim_eta = 0.0 if ddim_eta is None else float(ddim_eta)
+        if ddim_steps < 2:
+            raise ValueError(f"ddim_steps={ddim_steps}: the grid needs at least 2 points (one model evaluation)")
+        steps, flags = _ddim_plan(ddim_steps, False, np.inf)
+    elif ddim_steps is not None or ddim_eta is not None:
+        raise ValueError("ddim_steps / ddim_eta select the DDIM grid: they need use_ddim=True")
     dev = _pick_device(model, device)
     _io.seed_everything(seed)
     if x_T is None:
@@ -46,18 +62,28 @@ def get_samples(model, batch_size: int, seed: int, num_channels: int, sample_hei
     x = x.pin_memory().to(dev, non_blocking=True)
     with torch.cuda.device(dev):
         eng = model.engine(batch_size)
-        sampler = cached_sampler(eng, None, np.inf, batch_size, rule="predict_noise", ee_threshold=threshold,
-                                 ee_mode=mode)
+        rule = ("ddim", ddim_steps, ddim_eta) if use_ddim else "predict_noise"
+        sampler = cached_sampler(eng, None, np.inf, batch_size, rule=rule, ee_threshold=threshold, ee_mode=mode)
         sampler.set_noise_offset(noise_row_offset)
         exit_log = torch.zeros(1000, batch_size, device=dev, dtype=torch.int32)
         score_log = torch.zeros(1000, depth, device=dev, dtype=torch.float32)
         if noise is not None:
             noise = noise.to(device=dev, dtype=torch.float32).contiguous()
-        sampler.run(x, y=y, noise=noise, seed=seed, exit_log=exit_log, score_log=score_log, use_graph=use_graph)
+        if use_ddim:
+            sampler.run_list(x, steps, flags, y=y, noise=noise, seed=seed, exit_log=exit_log, score_log=score_log,
+                             use_graph=use_graph)
+        else:
+            sampler.run(x, y=y, noise=noise, seed=seed, exit_log=exit_log, score_log=score_log, use_graph=use_graph)
         if autoencoder:  # eesampler.py:84-85
             x = autoencoder.decode(x).contiguous()
         samples = sampler.finalize(x).cpu().numpy()
-    return samples, score_log.cpu(), exit_log.cpu().to(torch.float32)
+    score_log, exit_log = score_log.cpu(), exit_log.cpu().to(torch.float32)
+    if use_ddim:
+        off_grid = torch.ones(1000, dtype=torch.bool)
+        off_grid[steps] = False
+        score_log[off_grid] = float("nan")
+        exit_log[off_grid] = float("nan")
+    return samples, score_log, exit_log
 
 
 def dump_samples(samples, output_folder: Path):
@@ -84,7 +110,19 @@ def get_args(argv=None):
     p.add_argument("--output_folder", type=str, required=True)
     p.add_argument("--config_path", type=str, required=True, help="Path to yaml config file")
     p.add_argument("--class_id", type=int, default=None, help="Number up to 1000 that corresponds to a class")
-    return p.parse_args(argv)
+    # not flags of the reference's eesampler.py: absent from the namespace unless given, so DDPM runs parse as before
+    p.add_argument("--use_ddim", action="store_true", default=SUPPRESS,
+                   help="Sample on the strided DDIM grid of sampler.py --use_ddim, with early exit at every step")
+    p.add_argument("--ddim_steps", type=int, default=SUPPRESS, help="DDIM grid points (default 50; needs --use_ddim)")
+    p.add_argument("--ddim_eta", type=float, default=SUPPRESS, help="DDIM eta (default 0; needs --use_ddim)")
+    args = p.parse_args(argv)
+    if not getattr(args, "use_ddim", False):
+        for flag in ("ddim_steps", "ddim_eta"):
+            if hasattr(args, flag):
+                p.error(f"--{flag} needs --use_ddim")
+    elif getattr(args, "ddim_steps", 2) < 2:
+        p.error("--ddim_steps needs at least 2 grid points (one model evaluation)")
+    return args
 
 
 def main(argv=None):
@@ -112,13 +150,14 @@ def main(argv=None):
             y = draw_labels(args.batch_size, mp.get("num_classes", -1)).to(device)
         if "autoencoder" in cfg and hi > lo:  # eesampler.py:184-189
             autoencoder = get_autoencoder(cfg["autoencoder"]["autoencoder_checkpoint_path"])
+        extra = {k: getattr(args, k) for k in ("use_ddim", "ddim_steps", "ddim_eta") if hasattr(args, k)}
         D.barrier()  # every rank has loaded its model: the clock starts together
         tic = time.time()
         local = D.run_shard(
             functools.partial(get_samples, model=model), args.batch_size,
             shape=(mp["in_chans"], mp["img_size"], mp["img_size"]), seed=args.seed, y=y,
             num_channels=mp["in_chans"], sample_height=mp["img_size"], sample_width=mp["img_size"],
-            threshold=args.threshold, depth=mp["depth"], autoencoder=autoencoder)
+            threshold=args.threshold, depth=mp["depth"], autoencoder=autoencoder, **extra)
         D.barrier()  # every shard is done: what follows is the gather alone
         t_gather = time.time()
         result = D.gather_to_rank0(local, args.batch_size, D.EESAMPLER_OUTPUTS)

@@ -161,6 +161,14 @@ int ddb_sampler_run(ddb_sampler* s, float* x_dev, const int64_t* y_dev, const fl
 int ddb_sampler_run_list(ddb_sampler* s, float* x_dev, const int64_t* y_dev, const float* z_all_dev, uint64_t seed,
                          const int32_t* t_list_host, const uint8_t* late_host, int32_t n_steps, float* eps_trace_dev,
                          float* x_trace_dev, int32_t use_graph, void* stream);
+/* ddb_sampler_run_list with the early-exit logs of ddb_sampler_run: exit_idx_trace_dev [1000, B] i32 and
+ * score_mean_trace_dev [1000, depth] f32 (either may be NULL), indexed by t.  Only the rows of the timesteps in
+ * t_list are written; every other row keeps the caller's contents.  Used for DDIM sampling with early exit (step_mode
+ * 2, ee_mode >= 0).  Asking for a log from a sampler without early exit fails with DDB_ERR_INVALID. */
+int ddb_sampler_run_list_logs(ddb_sampler* s, float* x_dev, const int64_t* y_dev, const float* z_all_dev,
+                              uint64_t seed, const int32_t* t_list_host, const uint8_t* late_host, int32_t n_steps,
+                              float* eps_trace_dev, float* x_trace_dev, int32_t* exit_idx_trace_dev,
+                              float* score_mean_trace_dev, int32_t use_graph, void* stream);
 /* samples = (x + 1) / 2, NCHW -> NHWC (sampler.py:145-146). */
 int ddb_finalize_nhwc(const float* x_dev, float* out_dev, int32_t B, int32_t C, int32_t H, int32_t W, void* stream);
 /* Process-wide runtime switches for A/B measurements (DESIGN.md lists them): "alt_dir", "attn_discard", "pdl",
