@@ -1066,12 +1066,12 @@ static int launch_token_extras(const ddb_model* m, const float* t_vec, const int
     LAUNCH_CHECK();
     return DDB_OK;
 }
-template <bool G>
+template <bool G, int K>
 static void (*ms_tail_kernel(int C, int W))(TailArgs) {
-    if (C == 3 && W == 64) return step_tail_kernel<3, 64, G, true>;
-    if (C == 3 && W == 32) return step_tail_kernel<3, 32, G, true>;
-    if (C == 4 && W == 32) return step_tail_kernel<4, 32, G, true>;
-    if (C == 4 && W == 64) return step_tail_kernel<4, 64, G, true>;
+    if (C == 3 && W == 64) return step_tail_kernel<3, 64, G, K>;
+    if (C == 3 && W == 32) return step_tail_kernel<3, 32, G, K>;
+    if (C == 4 && W == 32) return step_tail_kernel<4, 32, G, K>;
+    if (C == 4 && W == 64) return step_tail_kernel<4, 64, G, K>;
     return nullptr;
 }
 // B: rows of the forward; a guided tail runs one CTA per guided sample (ta.B = B / 2) and band
@@ -1080,8 +1080,12 @@ static int launch_step_tail(const ddb_model* m, const TailArgs& ta, int B, cudaS
     const dim3 grid((ta.guide ? ta.B : B) * (H / CONV_BAND));
     ProfScope ps(PC_TAIL);
     if (ta.mode == 3) {  // DPM-Solver++(2M): the multistep instantiations, guided or not
-        void (*k)(TailArgs) = ta.guide ? ms_tail_kernel<true>(C, W) : ms_tail_kernel<false>(C, W);
+        void (*k)(TailArgs) = ta.guide ? ms_tail_kernel<true, TAIL_DPM2M>(C, W) : ms_tail_kernel<false, TAIL_DPM2M>(C, W);
         if (!k) return fail(DDB_ERR_INVALID, "sample shape [%d,%d,%d] unsupported by the multistep step tail", C, H, W);
+        CUDA_TRY(launch_pdl(k, grid, dim3(256), 0, st, ta));
+    } else if (ta.mode == 4) {  // UniPC: the predictor-corrector instantiations, guided or not
+        void (*k)(TailArgs) = ta.guide ? ms_tail_kernel<true, TAIL_UNIPC>(C, W) : ms_tail_kernel<false, TAIL_UNIPC>(C, W);
+        if (!k) return fail(DDB_ERR_INVALID, "sample shape [%d,%d,%d] unsupported by the UniPC step tail", C, H, W);
         CUDA_TRY(launch_pdl(k, grid, dim3(256), 0, st, ta));
     } else if (ta.guide) {
         if (C == 3 && W == 64)
@@ -1472,6 +1476,9 @@ struct ddb_sampler {
     // starts a new history), and the order column of the table (0: no step starts at t)
     Buf d_prev;
     std::vector<float> ms_order;
+    // UniPC (step_mode 4): d_prev holds D1; D2 and the corrected x of the previous step, kept across runs like d_prev
+    // (a corrector-0 row starts a new history).  ms_order is the predictor order column
+    Buf d_prev2, x_base;
     bool early_exit() const { return ee_mode >= 0 && early->cfg.early_exit; }
     // every step ends in step_tail_kernel, which also prepares the head of the next step (plain backbones always;
     // early exit in compaction mode on the CTA-pair path, option "ee_fuse")
@@ -1554,6 +1561,8 @@ static int sampler_step(ddb_sampler* s, ddb_model* m, float* x, bool has_y, cons
     tail_target(ta.tgt[1], s->late ? s->late : s->early);
     ta.guide = s->guide, ta.scale = s->cfg_scale, ta.B = B;
     ta.d_prev = s->d_prev ? s->d_prev->as<float>() : nullptr;
+    ta.d_prev2 = s->d_prev2 ? s->d_prev2->as<float>() : nullptr;
+    ta.x_base = s->x_base ? s->x_base->as<float>() : nullptr;
     if (s->guide) return forward_impl(m, x, nullptr, y, 2 * B, nullptr, false, st, nullptr, &f);
     if (ee_on) {
         // early exit with compaction: the same fused step; the tail picks every sample's conv weights by its exit layer
@@ -1723,6 +1732,9 @@ int ddb_ddpm_step(float* x_dev, const float* model_out_dev, const float* z_dev, 
     if (mode == 3)
         return fail(DDB_ERR_INVALID, "mode 3 (DPM-Solver++) needs the previous step's data prediction: run it "
                                      "through a sampler");
+    if (mode == 4)
+        return fail(DDB_ERR_INVALID, "mode 4 (UniPC) needs the previous steps' data predictions: run it through a "
+                                     "sampler");
     // z_dev is this step's tensor: stride 0 makes z_all + t*stride land on it
     ddpm_step_kernel<<<(unsigned)((n / 4 + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
         x_dev, model_out_dev, z_dev, (size_t)n, (size_t)0, coef_dev, nullptr, t, mode, seed, nullptr, nullptr);
@@ -1740,20 +1752,27 @@ int ddb_sampler_create(ddb_model* early, ddb_model* late, int32_t switch_t, int3
     if (ee_mode < -1 || ee_mode > 1) return fail(DDB_ERR_INVALID, "ee_mode must be -1 (off), 0 (simulate) or 1 (compact)");
     if (ee_mode >= 0 && !early->cfg.early_exit)
         return fail(DDB_ERR_INVALID, "early exit requested but the model was not created with early_exit=1");
-    if (step_mode < 0 || step_mode > 3) return fail(DDB_ERR_INVALID, "step_mode must be 0, 1, 2 or 3");
+    if (step_mode < 0 || step_mode > 4) return fail(DDB_ERR_INVALID, "step_mode must be 0, 1, 2, 3 or 4");
     if (step_mode == 3 && ee_mode >= 0)
         return fail(DDB_ERR_INVALID, "step_mode 3 (DPM-Solver++) is not supported with early exit");
+    if (step_mode == 4 && ee_mode >= 0)
+        return fail(DDB_ERR_INVALID, "step_mode 4 (UniPC) is not supported with early exit");
     std::unique_ptr<ddb_sampler> s(new ddb_sampler());
     s->early = early, s->late = late, s->switch_t = switch_t, s->B = B, s->step_mode = step_mode;
     s->ee_threshold = ee_threshold, s->ee_mode = ee_mode;
     s->n = (size_t)B * early->chw;
-    const int row = step_mode == 3 ? 8 : 4;  // floats per timestep of the coefficient table
+    const int row = step_mode == 4 ? 12 : step_mode == 3 ? 8 : 4;  // floats per timestep of the coefficient table
     DDB_TRY(new_buf(s->coef, (size_t)1000 * row * 4));
     CUDA_TRY(cudaMemcpy(s->coef->p, coef_host, (size_t)1000 * row * 4, cudaMemcpyHostToDevice));
-    if (step_mode == 3) {
+    if (step_mode >= 3) {
         DDB_TRY(new_buf(s->d_prev, s->n * 4));
         s->ms_order.resize(1000);
-        for (int t = 0; t < 1000; ++t) s->ms_order[t] = coef_host[t * 8 + 6];
+        const int col = step_mode == 4 ? 10 : 6;  // the (predictor) order column
+        for (int t = 0; t < 1000; ++t) s->ms_order[t] = coef_host[t * row + col];
+    }
+    if (step_mode == 4) {
+        DDB_TRY(new_buf(s->d_prev2, s->n * 4));
+        DDB_TRY(new_buf(s->x_base, s->n * 4));
     }
     DDB_TRY(new_buf(s->t_dev, 4));
     DDB_TRY(new_buf(s->t_vec, (size_t)B * 4));
@@ -1824,6 +1843,9 @@ static int sampler_run_impl(ddb_sampler* s, float* x_dev, const int64_t* y_dev, 
         if (late[k] && !s->late) return fail(DDB_ERR_INVALID, "step %d asks for the late model but none was given", k);
         if (s->step_mode == 3 && s->ms_order[t_list[k]] == 0.f)
             return fail(DDB_ERR_INVALID, "timestep %d is not a step of the DPM-Solver++ grid (order 0 in the table)",
+                        t_list[k]);
+        if (s->step_mode == 4 && s->ms_order[t_list[k]] == 0.f)
+            return fail(DDB_ERR_INVALID, "timestep %d is not a step of the UniPC grid (predictor order 0 in the table)",
                         t_list[k]);
     }
     if (use_graph && (eps_trace_dev || x_trace_dev))
@@ -1944,6 +1966,8 @@ int ddb_sampler_run(ddb_sampler* s, float* x_dev, const int64_t* y_dev, const fl
     if (t_first > 999 || t_last < 0 || t_last > t_first) return fail(DDB_ERR_INVALID, "bad step range");
     if (s->step_mode == 3)
         return fail(DDB_ERR_INVALID, "DPM-Solver++ (step_mode 3) runs over its grid only: use ddb_sampler_run_list");
+    if (s->step_mode == 4)
+        return fail(DDB_ERR_INVALID, "UniPC (step_mode 4) runs over its grid only: use ddb_sampler_run_list");
     std::vector<int32_t> ts;
     std::vector<uint8_t> late;
     for (int t = t_first; t >= t_last; --t) {

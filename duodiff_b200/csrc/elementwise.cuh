@@ -452,6 +452,28 @@ __device__ __forceinline__ float4 ms_update4(const MsCoef& k, bool second, float
     return make_float4(ms_update1(k, second, x.x, e.x, dp.x, dt.x), ms_update1(k, second, x.y, e.y, dp.y, dt.y),
                        ms_update1(k, second, x.z, e.z, dp.z, dt.z), ms_update1(k, second, x.w, e.w, dp.w, dt.w));
 }
+// UniPC (bh2, data prediction), mode 4 (ddpm.unipc_coefficients): row {a, b, cx, c0 | c1, c2, px, p0 | p1, corr,
+// pred, 0}.  No noise term.  With the history of the sampler (xb = corrected x of the previous step, D1 / D2 = the
+// data predictions of the previous two steps):
+//   D  = a*x + b*out
+//   corrector  xc = x (corr 0);  ((cx*xb + c0*D) + c1*D1) (corr 1);  (((cx*xb + c0*D) + c1*D1) + c2*D2) (corr 2)
+//   predictor  x' = px*xc + p0*D (pred 1);  (px*xc + p0*D) + p1*D1 (pred 2)
+// then xb <- xc, D2 <- D1, D1 <- D.  Every operation rounded on its own.  The order columns decide what is read: a
+// corrector-0 row reads no history and a corrector-1 row does not read D2 (NaN * 0 would still be NaN).
+struct UniCoef {
+    float a, b, cx, c0, c1, c2, px, p0, p1;
+};
+__device__ __forceinline__ float unipc_update1(const UniCoef& k, int corr, int pred, float x, float e, float xb,
+                                               float d1, float d2, float& d, float& xc) {
+    d = __fadd_rn(__fmul_rn(k.a, x), __fmul_rn(k.b, e));
+    xc = x;
+    if (corr >= 1) {
+        xc = __fadd_rn(__fadd_rn(__fmul_rn(k.cx, xb), __fmul_rn(k.c0, d)), __fmul_rn(k.c1, d1));
+        if (corr == 2) xc = __fadd_rn(xc, __fmul_rn(k.c2, d2));
+    }
+    const float o = __fadd_rn(__fmul_rn(k.px, xc), __fmul_rn(k.p0, d));
+    return pred == 2 ? __fadd_rn(o, __fmul_rn(k.p1, d1)) : o;
+}
 
 // seed_dev (graph replay / sampler): {Philox key, float4 index of this shard's first element in the global batch}
 __global__ void __launch_bounds__(256) ddpm_step_kernel(float* __restrict__ x, const float* __restrict__ model_out,
@@ -502,7 +524,7 @@ struct TailArgs {
     const float* conv_b;
     float* x;              // [B,C,H,W] in place
     const float* z_all;    // injected noise [1000, n] or null (Philox)
-    const float* coef;     // [1000,4]; mode 3 (DPM-Solver++): [1000,8]
+    const float* coef;     // [1000,4]; mode 3 (DPM-Solver++): [1000,8]; mode 4 (UniPC): [1000,12]
     int* t_dev;            // step counter (read by every CTA, advanced by the last one to finish)
     const int* next_t;     // [1000] successor table; [1000, 2000): 1 = the step after t runs on the late backbone
     const unsigned long long* seed_dev;  // {Philox key, float4 offset of the shard in the global batch}
@@ -525,17 +547,26 @@ struct TailArgs {
     int guide;             // 0 / 1; selects the G = true instantiation on the host
     float scale;
     int B;                 // guided samples (x, noise and traces have B rows)
-    // DPM-Solver++(2M) (mode 3, MS = true): the previous step's data prediction D_prev [B,C,H,W], sampler-owned
+    // DPM-Solver++(2M) (mode 3, K = TAIL_DPM2M): the previous step's data prediction D_prev [B,C,H,W], sampler-owned
     float* d_prev;
+    // UniPC (mode 4, K = TAIL_UNIPC): d_prev is D1; the data prediction of the step before it, D2, and the corrected
+    // x of the previous step, xb [B,C,H,W] each, sampler-owned
+    float* d_prev2;
+    float* x_base;
 };
+// the update a step_tail_kernel instantiation applies: DDPM / DDIM (modes 0-2), DPM-Solver++(2M) (mode 3), UniPC (4)
+enum TailKind { TAIL_DDPM = 0, TAIL_DPM2M = 1, TAIL_UNIPC = 2 };
 // G = true: the guided tail (one CTA per guided sample b and band).  It stages two bands, rows b and b + B of img_pre,
 // one after the other so that the staging needs the registers of one band; shared memory doubles (C = 4, W = 64:
 // 43008 B per CTA by -Xptxas -v, so 4 CTAs still fit an SM).  G = false compiles to the same SASS as before.
-// MS = true: the multistep update of mode 3 (ms_update4) replaces the DDPM / DDIM one; it reads the 8-float row as two
-// float4 and D_prev (order-2 rows only) at the element the thread owns, and writes D_t there.  MS = false compiles to
-// the same SASS as before.
-template <int C, int W, bool G = false, bool MS = false>
+// K = TAIL_DPM2M: the multistep update of mode 3 (ms_update4) replaces the DDPM / DDIM one; it reads the 8-float row
+// as two float4 and D_prev (order-2 rows only) at the element the thread owns, and writes D_t there.
+// K = TAIL_UNIPC: the predictor-corrector update of mode 4 (unipc_update1); it reads the 12-float row as three float4,
+// and xb, D1 (corrector order >= 1) and D2 (order 2) at the element the thread owns, and writes xb, D1 and D2 there:
+// 24 B per element more than the DDIM tail.  Both skip the noise.  K = TAIL_DDPM compiles to the same SASS as before.
+template <int C, int W, bool G = false, int K = TAIL_DDPM>
 __global__ void __launch_bounds__(256, 4) step_tail_kernel(const __grid_constant__ TailArgs a) {
+    constexpr bool MS = K == TAIL_DPM2M, UP = K == TAIL_UNIPC;
     constexpr int SW = W + 8, SH = CONV_BAND + 2, w4 = W / 4;
     constexpr int N_ITEMS = C * CONV_BAND * w4;          // (output channel, row, 4-pixel group) work items
     constexpr int BAND = C * SH * SW;                    // floats of one staged band
@@ -558,9 +589,11 @@ __global__ void __launch_bounds__(256, 4) step_tail_kernel(const __grid_constant
     const int t = ld_state(a.t_dev);
     // everything that depends on t is requested at once (one further round trip, not three)
     const int t_next = a.next_t[t], late_next = a.next_t[1000 + t];
-    const float4 kc = *reinterpret_cast<const float4*>(a.coef + t * (MS ? 8 : 4));
-    float4 kc2;
-    if constexpr (MS) kc2 = *reinterpret_cast<const float4*>(a.coef + t * 8 + 4);
+    constexpr int ROW = UP ? 12 : (MS ? 8 : 4);
+    const float4 kc = *reinterpret_cast<const float4*>(a.coef + t * ROW);
+    float4 kc2, kc3;
+    if constexpr (MS || UP) kc2 = *reinterpret_cast<const float4*>(a.coef + t * ROW + 4);
+    if constexpr (UP) kc3 = *reinterpret_cast<const float4*>(a.coef + t * ROW + 8);
     const unsigned long long seed = ld_state(a.seed_dev), off4 = ld_state(a.seed_dev + 1);
     // band of the decoder image (guided: row b, then row b + B): all loads of a thread are in flight before its first
     // shared-memory store
@@ -597,9 +630,16 @@ __global__ void __launch_bounds__(256, 4) step_tail_kernel(const __grid_constant
         const size_t e4 = ((((size_t)b * C + co) * H + y0 + yy) * W) / 4 + xq;  // float4 index inside the shard
         // x (and the injected noise) do not depend on the conv: their loads are in flight while it is computed
         const float4 xv = reinterpret_cast<const float4*>(a.x)[e4];
-        float4 zv = make_float4(0.f, 0.f, 0.f, 0.f);  // MS: D_prev
+        float4 zv = make_float4(0.f, 0.f, 0.f, 0.f);  // MS: D_prev; UP: D1
+        float4 xb = zv, d2 = zv;                       // UP
         if constexpr (MS) {
             if (kc2.z == 2.f) zv = reinterpret_cast<const float4*>(a.d_prev)[e4];
+        } else if constexpr (UP) {
+            if (kc3.y != 0.f) {
+                zv = reinterpret_cast<const float4*>(a.d_prev)[e4];
+                xb = reinterpret_cast<const float4*>(a.x_base)[e4];
+            }
+            if (kc3.y == 2.f) d2 = reinterpret_cast<const float4*>(a.d_prev2)[e4];
         } else if (t > 0 && a.z_all) {
             zv = reinterpret_cast<const float4*>(a.z_all + (size_t)t * a.n)[e4];
         }
@@ -619,6 +659,17 @@ __global__ void __launch_bounds__(256, 4) step_tail_kernel(const __grid_constant
             float4 dt;
             o = ms_update4(MsCoef{kc.x, kc.y, kc.z, kc.w, kc2.x, kc2.y}, kc2.z == 2.f, xv, ev, zv, dt);
             reinterpret_cast<float4*>(a.d_prev)[e4] = dt;
+        } else if constexpr (UP) {
+            const UniCoef u{kc.x, kc.y, kc.z, kc.w, kc2.x, kc2.y, kc2.z, kc2.w, kc3.x};
+            const int corr = (int)kc3.y, pred = (int)kc3.z;
+            float4 d, xc;
+            o.x = unipc_update1(u, corr, pred, xv.x, ev.x, xb.x, zv.x, d2.x, d.x, xc.x);
+            o.y = unipc_update1(u, corr, pred, xv.y, ev.y, xb.y, zv.y, d2.y, d.y, xc.y);
+            o.z = unipc_update1(u, corr, pred, xv.z, ev.z, xb.z, zv.z, d2.z, d.z, xc.z);
+            o.w = unipc_update1(u, corr, pred, xv.w, ev.w, xb.w, zv.w, d2.w, d.w, xc.w);
+            reinterpret_cast<float4*>(a.x_base)[e4] = xc;
+            if (corr != 0) reinterpret_cast<float4*>(a.d_prev2)[e4] = zv;
+            reinterpret_cast<float4*>(a.d_prev)[e4] = d;
         } else {
             if (t > 0 && !a.z_all) zv = philox_normal4(e4 + off4, t, seed);
             o = ddpm_update4(a.mode, k, xv, ev, zv);

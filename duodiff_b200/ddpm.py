@@ -74,6 +74,71 @@ def dpm_solver_coefficients(steps: int, parametrization: str = "predict_noise"):
     return table.to(torch.float32).contiguous(), 3
 
 
+def _unipc_table64(steps: int, parametrization: str = "predict_noise") -> torch.Tensor:
+    """The [1000,12] table of unipc_coefficients in fp64, before its single rounding to fp32."""
+    if parametrization not in ("predict_noise", "predict_original"):
+        raise ValueError(f"UniPC needs a data or noise prediction, not {parametrization!r}")
+    if int(steps) < 2:
+        raise ValueError(f"unipc_steps={steps}: the grid needs at least 2 points (one model evaluation)")
+    ab = schedule()["alphas_bar"].double()
+    alpha, sigma = ab.sqrt(), (1 - ab).sqrt()
+    lam = [float(v) for v in alpha.log() - sigma.log()]
+    alpha, sigma = [float(v) for v in alpha], [float(v) for v in sigma]
+    ts = ddim_timesteps(int(steps))
+    evals = len(ts) - 1
+    order = [1 if k == 0 or k == evals - 1 else 2 for k in range(evals)]  # predictor order (lower_order_final)
+    table = torch.zeros(1000, 12, dtype=torch.float64)
+    for k in range(evals):
+        t, s = ts[k], ts[k + 1]
+        a, b = (0.0, 1.0) if parametrization == "predict_original" else (1 / alpha[t], -sigma[t] / alpha[t])
+        # corrector from the previous base point to t (order of the predictor that produced x at t)
+        cx = c0 = c1 = c2 = 0.0
+        corr = order[k - 1] if k > 0 else 0
+        if corr:
+            h = lam[t] - lam[ts[k - 1]]
+            phi = math.expm1(-h)
+            bh = phi  # B(h) of the bh2 variant
+            al = alpha[t]
+            cx = sigma[t] / sigma[ts[k - 1]]
+            if corr == 1:
+                c0 = -al * bh * 0.5
+                c1 = -al * phi + al * bh * 0.5
+            else:
+                r = (lam[ts[k - 2]] - lam[ts[k - 1]]) / h
+                g1 = phi / -h - 1
+                g2 = g1 / -h - 0.5
+                rho0 = (g1 / bh - 2 * g2 / bh) / (1 - r)  # [[1, 1], [r, 1]] [rho0, rho1] = [g1/B, 2 g2/B]
+                rho1 = g1 / bh - rho0
+                c0 = -al * bh * rho1
+                c1 = -al * phi + al * bh * rho0 / r + al * bh * rho1
+                c2 = -al * bh * rho0 / r
+        # predictor from the corrected x at t to s
+        h = lam[s] - lam[t]
+        phi = math.expm1(-h)
+        px, p0, p1 = sigma[s] / sigma[t], -alpha[s] * phi, 0.0
+        if order[k] == 2:
+            r = (lam[ts[k - 1]] - lam[t]) / h
+            p0 += alpha[s] * phi / (2 * r)
+            p1 = -alpha[s] * phi / (2 * r)
+        table[t] = torch.tensor([a, b, cx, c0, c1, c2, px, p0, p1, corr, order[k], 0.0], dtype=torch.float64)
+    return table
+
+
+def unipc_coefficients(steps: int, parametrization: str = "predict_noise"):
+    """[1000,12] fp32 table {a, b, cx, c0, c1, c2, px, p0, p1, corrector order, predictor order, 0} of UniPC (Zhao et
+    al., 2023: bh2, order 2, data prediction), mode 4 of the step kernel, over the DDIM grid ddim_timesteps(steps)
+    (steps - 1 model evaluations).  With alpha = sqrt(abar), sigma = sqrt(1 - abar), lambda = log(alpha / sigma), the
+    step that evaluates the model at x_k, t_k computes the data prediction D_k = a*x_k + b*out (predict_noise: a =
+    1/alpha, b = -sigma/alpha; predict_original: a = 0, b = 1), then
+        corrector  xc_k    = cx*xc_{k-1} + c0*D_k + c1*D_{k-1} + c2*D_{k-2}     (xc_0 = x_0: corrector order 0)
+        predictor  x_{k+1} = px*xc_k + p0*D_k + p1*D_{k-1}
+    The corrector, UniC, reuses this step's evaluation, so it costs no model call; its order is the order of the
+    predictor that produced x_k.  The predictor, UniP, is order 1 on the first and the final step (lower_order_final)
+    and 2 otherwise.  The structured form of both is oracle/unipc_oracle.py.  Computed in fp64 from the fp32 schedule,
+    rounded once.  Rows of timesteps no step starts from are zero (predictor order 0)."""
+    return _unipc_table64(steps, parametrization).to(torch.float32).contiguous(), 4
+
+
 def schedule() -> dict:
     """The five schedule vectors, built with the reference's own torch calls (sampler.py:40-44) on the host so the
     coefficient table is bit-identical to a CPU run of the reference."""
@@ -162,6 +227,8 @@ class Sampler:
             table, mode = ddim_coefficients(int(rule[1]), float(rule[2]))
         elif isinstance(rule, tuple) and rule[0] == "dpm_solver++":  # ("dpm_solver++", steps, parametrization)
             table, mode = dpm_solver_coefficients(int(rule[1]), rule[2])
+        elif isinstance(rule, tuple) and rule[0] == "unipc":  # ("unipc", steps, parametrization)
+            table, mode = unipc_coefficients(int(rule[1]), rule[2])
         else:
             table, mode = step_coefficients(rule, variance)
         self.coef = table

@@ -115,11 +115,26 @@ def _dpm_solver_rule(models, postprocessing, use_ddim, steps):
     return "dpm_solver++", int(steps), name
 
 
+def _unipc_rule(models, postprocessing, use_ddim, dpm_solver_steps, steps):
+    """Sampler rule ("unipc", steps, parametrization) of UniPC, checked against the run."""
+    from .early_exit import EarlyExitUViT
+    if use_ddim or dpm_solver_steps is not None:
+        raise ValueError("unipc_steps, use_ddim and dpm_solver_steps select different samplers: give one of them")
+    name = _rule_name(postprocessing)
+    if name == "predict_previous":
+        raise ValueError("UniPC needs a noise or data prediction, not predict_previous")
+    if int(steps) < 2:
+        raise ValueError(f"unipc_steps={steps}: the grid needs at least 2 points (one model evaluation)")
+    if any(isinstance(m, EarlyExitUViT) for m in models):
+        raise ValueError("unipc_steps is not supported with early exit")
+    return "unipc", int(steps), name
+
+
 def get_samples(model, batch_size: int, postprocessing, seed: int, num_channels: int, sample_height: int,
                 sample_width: int, use_ddim: bool = False, ddim_steps: int = 50, ddim_eta: float = 0.0,
                 timesteps_save: List[int] = (), y=None, autoencoder=None, late_model=None, t_switch=np.inf, *,
                 noise=None, use_graph: bool = True, device=None, x_T=None, noise_row_offset: int = 0,
-                cfg_scale=None, null_label=None, dpm_solver_steps=None):
+                cfg_scale=None, null_label=None, dpm_solver_steps=None, unipc_steps=None):
     """sampler.py:82-155.  Returns (samples [B,H,W,C] f32 numpy un-clipped, [intermediate samples]).
 
     x_T is drawn on the CPU generator after ``seed_everything(seed)`` exactly like the reference (sampler.py:99-100);
@@ -141,14 +156,21 @@ def get_samples(model, batch_size: int, postprocessing, seed: int, num_channels:
     DPM-Solver++(2M) (not in the reference): ``dpm_solver_steps`` n runs the second-order multistep solver of the
     probability-flow ODE over the DDIM grid (n - 1 model evaluations at the timesteps of ``use_ddim=True,
     ddim_steps=n``), with the hand-off, ``timesteps_save``, ``autoencoder`` and ``cfg_scale`` as in the DDIM branch.
-    It has no noise term.  ``postprocessing`` must be predict_noise or predict_original."""
+    It has no noise term.  ``postprocessing`` must be predict_noise or predict_original.
+
+    UniPC (not in the reference): ``unipc_steps`` n runs the second-order predictor-corrector solver of the same ODE
+    (bh2, data prediction) over the same grid and with the same options as ``dpm_solver_steps``.  The corrector reuses
+    each step's model evaluation, so n - 1 evaluations still suffice; the final step is first order.  A saved
+    intermediate is the predicted x the next evaluation sees (its correction needs that evaluation)."""
     models = [m for m in (model, late_model) if m is not None]
     guidance = None
     if cfg_scale is not None:
         guidance = _guidance(models, y, cfg_scale, null_label)
-    dpm_rule = None
+    solver_rule = None  # DPM-Solver++ or UniPC
     if dpm_solver_steps is not None:
-        dpm_rule = _dpm_solver_rule(models, postprocessing, use_ddim, dpm_solver_steps)
+        solver_rule = _dpm_solver_rule(models, postprocessing, use_ddim, dpm_solver_steps)
+    if unipc_steps is not None:
+        solver_rule = _unipc_rule(models, postprocessing, use_ddim, dpm_solver_steps, unipc_steps)
     dev = _pick_device(model, device)
     _io.seed_everything(seed)
     if x_T is None:
@@ -174,9 +196,9 @@ def get_samples(model, batch_size: int, postprocessing, seed: int, num_channels:
                 print("Decode the images...")
                 lat = autoencoder.decode(lat).contiguous()
             return sampler.finalize(lat)
-        if use_ddim or dpm_rule is not None:
-            # DDIM and DPM-Solver++ walk the same grid; after the step at t in save_at x is saved
-            rule = dpm_rule or ("ddim", int(ddim_steps), float(ddim_eta))
+        if use_ddim or solver_rule is not None:
+            # DDIM, DPM-Solver++ and UniPC walk the same grid; after the step at t in save_at x is saved
+            rule = solver_rule or ("ddim", int(ddim_steps), float(ddim_eta))
             sampler = cached_sampler(early, late, t_switch, batch_size, rule=rule, guidance=guidance)
             sampler.set_noise_offset(noise_row_offset)
             steps, flags = _ddim_plan(rule[1], late is not None, t_switch)
@@ -245,6 +267,9 @@ def get_args(argv=None):
     p.add_argument("--dpm_solver_steps", type=int, default=SUPPRESS,
                    help="Sample with DPM-Solver++(2M) over the DDIM grid of N points (N - 1 model evaluations, the "
                         "timesteps of --use_ddim --ddim_steps N); no noise term")
+    p.add_argument("--unipc_steps", type=int, default=SUPPRESS,
+                   help="Sample with UniPC (bh2, second-order predictor-corrector) over the DDIM grid of N points (N - 1 "
+                        "model evaluations, the timesteps of --use_ddim --ddim_steps N); no noise term")
     args = p.parse_args(argv)
     if getattr(args, "cfg_scale", None) is not None and args.class_id is None:
         p.error("--cfg_scale needs --class_id: guidance contrasts the class labels with the null label")
@@ -255,6 +280,13 @@ def get_args(argv=None):
             p.error("--dpm_solver_steps needs --parametrization predict_noise or predict_original")
         if args.dpm_solver_steps < 2:
             p.error("--dpm_solver_steps needs at least 2 grid points (one model evaluation)")
+    if getattr(args, "unipc_steps", None) is not None:
+        if args.use_ddim or getattr(args, "dpm_solver_steps", None) is not None:
+            p.error("--unipc_steps, --use_ddim and --dpm_solver_steps select different samplers: give one of them")
+        if args.parametrization == "predict_previous":
+            p.error("--unipc_steps needs --parametrization predict_noise or predict_original")
+        if args.unipc_steps < 2:
+            p.error("--unipc_steps needs at least 2 grid points (one model evaluation)")
     return args
 
 
@@ -308,6 +340,8 @@ def main(argv=None):
                       f"(the last row of the {mp.get('num_classes', -1)}-row label table)")
         if getattr(args, "dpm_solver_steps", None) is not None:
             extra["dpm_solver_steps"] = args.dpm_solver_steps
+        if getattr(args, "unipc_steps", None) is not None:
+            extra["unipc_steps"] = args.unipc_steps
         if "autoencoder" in cfg and hi > lo:  # sampler.py:320-325
             autoencoder = get_autoencoder(cfg["autoencoder"]["autoencoder_checkpoint_path"])
         D.barrier()  # every rank has loaded its models: the clock starts together
