@@ -1087,6 +1087,11 @@ static int launch_step_tail(const ddb_model* m, const TailArgs& ta, int B, cudaS
         void (*k)(TailArgs) = ta.guide ? ms_tail_kernel<true, TAIL_UNIPC>(C, W) : ms_tail_kernel<false, TAIL_UNIPC>(C, W);
         if (!k) return fail(DDB_ERR_INVALID, "sample shape [%d,%d,%d] unsupported by the UniPC step tail", C, H, W);
         CUDA_TRY(launch_pdl(k, grid, dim3(256), 0, st, ta));
+    } else if (ta.mode == 5) {  // SDE-DPM-Solver++(2M): the stochastic multistep instantiations, guided or not
+        void (*k)(TailArgs) = ta.guide ? ms_tail_kernel<true, TAIL_SDE2M>(C, W) : ms_tail_kernel<false, TAIL_SDE2M>(C, W);
+        if (!k)
+            return fail(DDB_ERR_INVALID, "sample shape [%d,%d,%d] unsupported by the SDE-DPM-Solver++ step tail", C, H, W);
+        CUDA_TRY(launch_pdl(k, grid, dim3(256), 0, st, ta));
     } else if (ta.guide) {
         if (C == 3 && W == 64)
             CUDA_TRY(launch_pdl(step_tail_kernel<3, 64, true>, grid, dim3(256), 0, st, ta));
@@ -1472,8 +1477,9 @@ struct ddb_sampler {
     // classifier-free guidance (ddb_sampler_set_guidance): every forward runs on 2B rows, y_buf holds [y ; null...]
     int guide = 0;
     float cfg_scale = 0.f;
-    // DPM-Solver++(2M) (step_mode 3): the previous step's data prediction [B,C,H,W], kept across runs (an order-1 row
-    // starts a new history), and the order column of the table (0: no step starts at t)
+    // DPM-Solver++(2M) (step_mode 3) and SDE-DPM-Solver++(2M) (step_mode 5): the previous step's data prediction
+    // [B,C,H,W], kept across runs (an order-1 row starts a new history), and the order column of the table (0: no
+    // step starts at t)
     Buf d_prev;
     std::vector<float> ms_order;
     // UniPC (step_mode 4): d_prev holds D1; D2 and the corrected x of the previous step, kept across runs like d_prev
@@ -1735,6 +1741,9 @@ int ddb_ddpm_step(float* x_dev, const float* model_out_dev, const float* z_dev, 
     if (mode == 4)
         return fail(DDB_ERR_INVALID, "mode 4 (UniPC) needs the previous steps' data predictions: run it through a "
                                      "sampler");
+    if (mode == 5)
+        return fail(DDB_ERR_INVALID, "mode 5 (SDE-DPM-Solver++) needs the previous step's data prediction: run it "
+                                     "through a sampler");
     // z_dev is this step's tensor: stride 0 makes z_all + t*stride land on it
     ddpm_step_kernel<<<(unsigned)((n / 4 + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
         x_dev, model_out_dev, z_dev, (size_t)n, (size_t)0, coef_dev, nullptr, t, mode, seed, nullptr, nullptr);
@@ -1752,16 +1761,18 @@ int ddb_sampler_create(ddb_model* early, ddb_model* late, int32_t switch_t, int3
     if (ee_mode < -1 || ee_mode > 1) return fail(DDB_ERR_INVALID, "ee_mode must be -1 (off), 0 (simulate) or 1 (compact)");
     if (ee_mode >= 0 && !early->cfg.early_exit)
         return fail(DDB_ERR_INVALID, "early exit requested but the model was not created with early_exit=1");
-    if (step_mode < 0 || step_mode > 4) return fail(DDB_ERR_INVALID, "step_mode must be 0, 1, 2, 3 or 4");
+    if (step_mode < 0 || step_mode > 5) return fail(DDB_ERR_INVALID, "step_mode must be 0, 1, 2, 3, 4 or 5");
     if (step_mode == 3 && ee_mode >= 0)
         return fail(DDB_ERR_INVALID, "step_mode 3 (DPM-Solver++) is not supported with early exit");
     if (step_mode == 4 && ee_mode >= 0)
         return fail(DDB_ERR_INVALID, "step_mode 4 (UniPC) is not supported with early exit");
+    if (step_mode == 5 && ee_mode >= 0)
+        return fail(DDB_ERR_INVALID, "step_mode 5 (SDE-DPM-Solver++) is not supported with early exit");
     std::unique_ptr<ddb_sampler> s(new ddb_sampler());
     s->early = early, s->late = late, s->switch_t = switch_t, s->B = B, s->step_mode = step_mode;
     s->ee_threshold = ee_threshold, s->ee_mode = ee_mode;
     s->n = (size_t)B * early->chw;
-    const int row = step_mode == 4 ? 12 : step_mode == 3 ? 8 : 4;  // floats per timestep of the coefficient table
+    const int row = step_mode == 4 ? 12 : step_mode >= 3 ? 8 : 4;  // floats per timestep of the coefficient table
     DDB_TRY(new_buf(s->coef, (size_t)1000 * row * 4));
     CUDA_TRY(cudaMemcpy(s->coef->p, coef_host, (size_t)1000 * row * 4, cudaMemcpyHostToDevice));
     if (step_mode >= 3) {
@@ -1847,6 +1858,9 @@ static int sampler_run_impl(ddb_sampler* s, float* x_dev, const int64_t* y_dev, 
         if (s->step_mode == 4 && s->ms_order[t_list[k]] == 0.f)
             return fail(DDB_ERR_INVALID, "timestep %d is not a step of the UniPC grid (predictor order 0 in the table)",
                         t_list[k]);
+        if (s->step_mode == 5 && s->ms_order[t_list[k]] == 0.f)
+            return fail(DDB_ERR_INVALID,
+                        "timestep %d is not a step of the SDE-DPM-Solver++ grid (order 0 in the table)", t_list[k]);
     }
     if (use_graph && (eps_trace_dev || x_trace_dev))
         return fail(DDB_ERR_INVALID, "per-step eps/x traces need use_graph=0");
@@ -1968,6 +1982,9 @@ int ddb_sampler_run(ddb_sampler* s, float* x_dev, const int64_t* y_dev, const fl
         return fail(DDB_ERR_INVALID, "DPM-Solver++ (step_mode 3) runs over its grid only: use ddb_sampler_run_list");
     if (s->step_mode == 4)
         return fail(DDB_ERR_INVALID, "UniPC (step_mode 4) runs over its grid only: use ddb_sampler_run_list");
+    if (s->step_mode == 5)
+        return fail(DDB_ERR_INVALID,
+                    "SDE-DPM-Solver++ (step_mode 5) runs over its grid only: use ddb_sampler_run_list");
     std::vector<int32_t> ts;
     std::vector<uint8_t> late;
     for (int t = t_first; t >= t_last; --t) {

@@ -452,6 +452,14 @@ __device__ __forceinline__ float4 ms_update4(const MsCoef& k, bool second, float
     return make_float4(ms_update1(k, second, x.x, e.x, dp.x, dt.x), ms_update1(k, second, x.y, e.y, dp.y, dt.y),
                        ms_update1(k, second, x.z, e.z, dp.z, dt.z), ms_update1(k, second, x.w, e.w, dp.w, dt.w));
 }
+// SDE-DPM-Solver++(2M), mode 5 (ddpm.sde_dpm_solver_coefficients): row {a, b, rho, phi | w0, w1, order, vs}.  The
+// update of mode 3 with rho = (sigma_s/sigma_t) exp(-h), phi = alpha_s (-expm1(-2h)), then the noise term:
+//   x' = (rho*x + phi*D) + vs*z      (vs = sigma_s sqrt(-expm1(-2h)); 0 on the final step, which adds nothing)
+// z is the DDPM tail's draw at t (Philox at (seed, t, global float4 index), or the injected z_all[t]).
+__device__ __forceinline__ float4 add_noise4(float4 o, float vs, float4 z) {
+    return make_float4(__fadd_rn(o.x, __fmul_rn(vs, z.x)), __fadd_rn(o.y, __fmul_rn(vs, z.y)),
+                       __fadd_rn(o.z, __fmul_rn(vs, z.z)), __fadd_rn(o.w, __fmul_rn(vs, z.w)));
+}
 // UniPC (bh2, data prediction), mode 4 (ddpm.unipc_coefficients): row {a, b, cx, c0 | c1, c2, px, p0 | p1, corr,
 // pred, 0}.  No noise term.  With the history of the sampler (xb = corrected x of the previous step, D1 / D2 = the
 // data predictions of the previous two steps):
@@ -524,7 +532,7 @@ struct TailArgs {
     const float* conv_b;
     float* x;              // [B,C,H,W] in place
     const float* z_all;    // injected noise [1000, n] or null (Philox)
-    const float* coef;     // [1000,4]; mode 3 (DPM-Solver++): [1000,8]; mode 4 (UniPC): [1000,12]
+    const float* coef;     // [1000,4]; modes 3 and 5 (DPM-Solver++, SDE): [1000,8]; mode 4 (UniPC): [1000,12]
     int* t_dev;            // step counter (read by every CTA, advanced by the last one to finish)
     const int* next_t;     // [1000] successor table; [1000, 2000): 1 = the step after t runs on the late backbone
     const unsigned long long* seed_dev;  // {Philox key, float4 offset of the shard in the global batch}
@@ -547,15 +555,17 @@ struct TailArgs {
     int guide;             // 0 / 1; selects the G = true instantiation on the host
     float scale;
     int B;                 // guided samples (x, noise and traces have B rows)
-    // DPM-Solver++(2M) (mode 3, K = TAIL_DPM2M): the previous step's data prediction D_prev [B,C,H,W], sampler-owned
+    // DPM-Solver++(2M) (mode 3, K = TAIL_DPM2M) and its SDE form (mode 5, K = TAIL_SDE2M): the previous step's data
+    // prediction D_prev [B,C,H,W], sampler-owned
     float* d_prev;
     // UniPC (mode 4, K = TAIL_UNIPC): d_prev is D1; the data prediction of the step before it, D2, and the corrected
     // x of the previous step, xb [B,C,H,W] each, sampler-owned
     float* d_prev2;
     float* x_base;
 };
-// the update a step_tail_kernel instantiation applies: DDPM / DDIM (modes 0-2), DPM-Solver++(2M) (mode 3), UniPC (4)
-enum TailKind { TAIL_DDPM = 0, TAIL_DPM2M = 1, TAIL_UNIPC = 2 };
+// the update a step_tail_kernel instantiation applies: DDPM / DDIM (modes 0-2), DPM-Solver++(2M) (mode 3), UniPC (4),
+// SDE-DPM-Solver++(2M) (5)
+enum TailKind { TAIL_DDPM = 0, TAIL_DPM2M = 1, TAIL_UNIPC = 2, TAIL_SDE2M = 3 };
 // G = true: the guided tail (one CTA per guided sample b and band).  It stages two bands, rows b and b + B of img_pre,
 // one after the other so that the staging needs the registers of one band; shared memory doubles (C = 4, W = 64:
 // 43008 B per CTA by -Xptxas -v, so 4 CTAs still fit an SM).  G = false compiles to the same SASS as before.
@@ -564,9 +574,11 @@ enum TailKind { TAIL_DDPM = 0, TAIL_DPM2M = 1, TAIL_UNIPC = 2 };
 // K = TAIL_UNIPC: the predictor-corrector update of mode 4 (unipc_update1); it reads the 12-float row as three float4,
 // and xb, D1 (corrector order >= 1) and D2 (order 2) at the element the thread owns, and writes xb, D1 and D2 there:
 // 24 B per element more than the DDIM tail.  Both skip the noise.  K = TAIL_DDPM compiles to the same SASS as before.
+// K = TAIL_SDE2M: the update of TAIL_DPM2M plus vs*z (mode 5).  It branches on vs, so the final step (vs = 0) neither
+// reads z_all nor runs Philox; the draw and the injected-noise index are the DDPM branch's, so sharding stays exact.
 template <int C, int W, bool G = false, int K = TAIL_DDPM>
 __global__ void __launch_bounds__(256, 4) step_tail_kernel(const __grid_constant__ TailArgs a) {
-    constexpr bool MS = K == TAIL_DPM2M, UP = K == TAIL_UNIPC;
+    constexpr bool SDE = K == TAIL_SDE2M, MS = K == TAIL_DPM2M || SDE, UP = K == TAIL_UNIPC;
     constexpr int SW = W + 8, SH = CONV_BAND + 2, w4 = W / 4;
     constexpr int N_ITEMS = C * CONV_BAND * w4;          // (output channel, row, 4-pixel group) work items
     constexpr int BAND = C * SH * SW;                    // floats of one staged band
@@ -632,8 +644,11 @@ __global__ void __launch_bounds__(256, 4) step_tail_kernel(const __grid_constant
         const float4 xv = reinterpret_cast<const float4*>(a.x)[e4];
         float4 zv = make_float4(0.f, 0.f, 0.f, 0.f);  // MS: D_prev; UP: D1
         float4 xb = zv, d2 = zv;                       // UP
+        float4 nz = zv;                                // SDE: this step's noise
         if constexpr (MS) {
             if (kc2.z == 2.f) zv = reinterpret_cast<const float4*>(a.d_prev)[e4];
+            if constexpr (SDE)
+                if (kc2.w != 0.f && a.z_all) nz = reinterpret_cast<const float4*>(a.z_all + (size_t)t * a.n)[e4];
         } else if constexpr (UP) {
             if (kc3.y != 0.f) {
                 zv = reinterpret_cast<const float4*>(a.d_prev)[e4];
@@ -658,6 +673,12 @@ __global__ void __launch_bounds__(256, 4) step_tail_kernel(const __grid_constant
         if constexpr (MS) {
             float4 dt;
             o = ms_update4(MsCoef{kc.x, kc.y, kc.z, kc.w, kc2.x, kc2.y}, kc2.z == 2.f, xv, ev, zv, dt);
+            if constexpr (SDE) {
+                if (kc2.w != 0.f) {
+                    if (!a.z_all) nz = philox_normal4(e4 + off4, t, seed);
+                    o = add_noise4(o, kc2.w, nz);
+                }
+            }
             reinterpret_cast<float4*>(a.d_prev)[e4] = dt;
         } else if constexpr (UP) {
             const UniCoef u{kc.x, kc.y, kc.z, kc.w, kc2.x, kc2.y, kc2.z, kc2.w, kc3.x};

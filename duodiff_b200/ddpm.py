@@ -139,6 +139,50 @@ def unipc_coefficients(steps: int, parametrization: str = "predict_noise"):
     return _unipc_table64(steps, parametrization).to(torch.float32).contiguous(), 4
 
 
+def _sde_dpm_solver_table64(steps: int, parametrization: str = "predict_noise") -> torch.Tensor:
+    """The [1000,8] table of sde_dpm_solver_coefficients in fp64, before its single rounding to fp32."""
+    if parametrization not in ("predict_noise", "predict_original"):
+        raise ValueError(f"SDE-DPM-Solver++ needs a data or noise prediction, not {parametrization!r}")
+    if int(steps) < 2:
+        raise ValueError(f"sde_dpm_solver_steps={steps}: the grid needs at least 2 points (one model evaluation)")
+    ab = schedule()["alphas_bar"].double()
+    alpha, sigma = ab.sqrt(), (1 - ab).sqrt()
+    lam = [float(v) for v in alpha.log() - sigma.log()]
+    alpha, sigma = [float(v) for v in alpha], [float(v) for v in sigma]
+    ts = ddim_timesteps(int(steps))
+    evals = len(ts) - 1
+    table = torch.zeros(1000, 8, dtype=torch.float64)
+    for k, (t, s) in enumerate(zip(ts[:-1], ts[1:])):
+        h = lam[s] - lam[t]
+        order = 1 if k == 0 or k == evals - 1 else 2
+        w0, w1 = 1.0, 0.0
+        if order == 2:
+            r = (lam[t] - lam[ts[k - 1]]) / h
+            w0, w1 = 1 + 1 / (2 * r), -1 / (2 * r)
+        a, b = (0.0, 1.0) if parametrization == "predict_original" else (1 / alpha[t], -sigma[t] / alpha[t])
+        e2 = -math.expm1(-2 * h)
+        vs = sigma[s] * math.sqrt(e2) if s > 0 else 0.0
+        table[t] = torch.tensor([a, b, sigma[s] / sigma[t] * math.exp(-h), alpha[s] * e2, w0, w1, order, vs],
+                                dtype=torch.float64)
+    return table
+
+
+def sde_dpm_solver_coefficients(steps: int, parametrization: str = "predict_noise"):
+    """[1000,8] fp32 table {a, b, rho, phi, w0, w1, order, vs} of SDE-DPM-Solver++(2M) (Lu et al., 2022: the
+    second-order multistep solver of the reverse SDE, data prediction), mode 5 of the step kernel, over the DDIM grid
+    ddim_timesteps(steps) (steps - 1 model evaluations).  With alpha = sqrt(abar), sigma = sqrt(1 - abar), lambda =
+    log(alpha / sigma), the step from t to the next grid point s, h = lambda_s - lambda_t, r = h_prev / h:
+        D_t = a*x + b*out            predict_noise: a = 1/alpha_t, b = -sigma_t/alpha_t;  predict_original: a = 0, b = 1
+        D   = w0*D_t + w1*D_prev     order 2: w0 = 1 + 1/(2r), w1 = -1/(2r);  order 1: D = D_t (w0 = 1, w1 = 0)
+        x'  = rho*x + phi*D + vs*z   rho = (sigma_s/sigma_t) exp(-h), phi = alpha_s (-expm1(-2h)),
+                                     vs = sigma_s sqrt(-expm1(-2h)) (0 on the final step, s = 0);  D_prev <- D_t
+    z is the draw of the DDPM step at t.  A first-order step is the DDPM posterior (ancestral) step from t to s; for s =
+    t - 1 it is the reference's DDPM update.  The first and the final step are order 1, the others order 2.  The
+    textbook form is oracle/sde_dpm_solver_oracle.py.  Computed in fp64 from the fp32 schedule, rounded once.  Rows of
+    timesteps no step starts from are zero (order 0)."""
+    return _sde_dpm_solver_table64(steps, parametrization).to(torch.float32).contiguous(), 5
+
+
 def schedule() -> dict:
     """The five schedule vectors, built with the reference's own torch calls (sampler.py:40-44) on the host so the
     coefficient table is bit-identical to a CPU run of the reference."""
@@ -229,6 +273,8 @@ class Sampler:
             table, mode = dpm_solver_coefficients(int(rule[1]), rule[2])
         elif isinstance(rule, tuple) and rule[0] == "unipc":  # ("unipc", steps, parametrization)
             table, mode = unipc_coefficients(int(rule[1]), rule[2])
+        elif isinstance(rule, tuple) and rule[0] == "sde-dpm_solver++":  # ("sde-dpm_solver++", steps, parametrization)
+            table, mode = sde_dpm_solver_coefficients(int(rule[1]), rule[2])
         else:
             table, mode = step_coefficients(rule, variance)
         self.coef = table

@@ -130,11 +130,27 @@ def _unipc_rule(models, postprocessing, use_ddim, dpm_solver_steps, steps):
     return "unipc", int(steps), name
 
 
+def _sde_dpm_solver_rule(models, postprocessing, use_ddim, dpm_solver_steps, unipc_steps, steps):
+    """Sampler rule ("sde-dpm_solver++", steps, parametrization) of SDE-DPM-Solver++(2M), checked against the run."""
+    from .early_exit import EarlyExitUViT
+    if use_ddim or dpm_solver_steps is not None or unipc_steps is not None:
+        raise ValueError("sde_dpm_solver_steps, use_ddim, dpm_solver_steps and unipc_steps select different samplers: "
+                         "give one of them")
+    name = _rule_name(postprocessing)
+    if name == "predict_previous":
+        raise ValueError("SDE-DPM-Solver++ needs a noise or data prediction, not predict_previous")
+    if int(steps) < 2:
+        raise ValueError(f"sde_dpm_solver_steps={steps}: the grid needs at least 2 points (one model evaluation)")
+    if any(isinstance(m, EarlyExitUViT) for m in models):
+        raise ValueError("sde_dpm_solver_steps is not supported with early exit")
+    return "sde-dpm_solver++", int(steps), name
+
+
 def get_samples(model, batch_size: int, postprocessing, seed: int, num_channels: int, sample_height: int,
                 sample_width: int, use_ddim: bool = False, ddim_steps: int = 50, ddim_eta: float = 0.0,
                 timesteps_save: List[int] = (), y=None, autoencoder=None, late_model=None, t_switch=np.inf, *,
                 noise=None, use_graph: bool = True, device=None, x_T=None, noise_row_offset: int = 0,
-                cfg_scale=None, null_label=None, dpm_solver_steps=None, unipc_steps=None):
+                cfg_scale=None, null_label=None, dpm_solver_steps=None, unipc_steps=None, sde_dpm_solver_steps=None):
     """sampler.py:82-155.  Returns (samples [B,H,W,C] f32 numpy un-clipped, [intermediate samples]).
 
     x_T is drawn on the CPU generator after ``seed_everything(seed)`` exactly like the reference (sampler.py:99-100);
@@ -161,16 +177,25 @@ def get_samples(model, batch_size: int, postprocessing, seed: int, num_channels:
     UniPC (not in the reference): ``unipc_steps`` n runs the second-order predictor-corrector solver of the same ODE
     (bh2, data prediction) over the same grid and with the same options as ``dpm_solver_steps``.  The corrector reuses
     each step's model evaluation, so n - 1 evaluations still suffice; the final step is first order.  A saved
-    intermediate is the predicted x the next evaluation sees (its correction needs that evaluation)."""
+    intermediate is the predicted x the next evaluation sees (its correction needs that evaluation).
+
+    SDE-DPM-Solver++(2M) (not in the reference): ``sde_dpm_solver_steps`` n runs the second-order multistep solver of
+    the reverse SDE over the same grid and with the same options as ``dpm_solver_steps``.  Each step but the final one
+    adds noise, the draw the DDPM step at that t makes (``seed`` or ``noise[t]``); a first-order step is the DDPM
+    posterior step between the two grid points.  The first and the final step are first order.  A saved intermediate
+    is x after that step, its noise included."""
     models = [m for m in (model, late_model) if m is not None]
     guidance = None
     if cfg_scale is not None:
         guidance = _guidance(models, y, cfg_scale, null_label)
-    solver_rule = None  # DPM-Solver++ or UniPC
+    solver_rule = None  # DPM-Solver++, UniPC or SDE-DPM-Solver++
     if dpm_solver_steps is not None:
         solver_rule = _dpm_solver_rule(models, postprocessing, use_ddim, dpm_solver_steps)
     if unipc_steps is not None:
         solver_rule = _unipc_rule(models, postprocessing, use_ddim, dpm_solver_steps, unipc_steps)
+    if sde_dpm_solver_steps is not None:
+        solver_rule = _sde_dpm_solver_rule(models, postprocessing, use_ddim, dpm_solver_steps, unipc_steps,
+                                           sde_dpm_solver_steps)
     dev = _pick_device(model, device)
     _io.seed_everything(seed)
     if x_T is None:
@@ -197,7 +222,8 @@ def get_samples(model, batch_size: int, postprocessing, seed: int, num_channels:
                 lat = autoencoder.decode(lat).contiguous()
             return sampler.finalize(lat)
         if use_ddim or solver_rule is not None:
-            # DDIM, DPM-Solver++ and UniPC walk the same grid; after the step at t in save_at x is saved
+            # DDIM and the DPM-Solver++ / UniPC / SDE solvers walk the same grid; after the step at t in save_at x is
+            # saved
             rule = solver_rule or ("ddim", int(ddim_steps), float(ddim_eta))
             sampler = cached_sampler(early, late, t_switch, batch_size, rule=rule, guidance=guidance)
             sampler.set_noise_offset(noise_row_offset)
@@ -270,6 +296,10 @@ def get_args(argv=None):
     p.add_argument("--unipc_steps", type=int, default=SUPPRESS,
                    help="Sample with UniPC (bh2, second-order predictor-corrector) over the DDIM grid of N points (N - 1 "
                         "model evaluations, the timesteps of --use_ddim --ddim_steps N); no noise term")
+    p.add_argument("--sde_dpm_solver_steps", type=int, default=SUPPRESS,
+                   help="Sample with SDE-DPM-Solver++(2M), the stochastic second-order multistep solver, over the DDIM "
+                        "grid of N points (N - 1 model evaluations, the timesteps of --use_ddim --ddim_steps N); every "
+                        "step but the final one adds noise")
     args = p.parse_args(argv)
     if getattr(args, "cfg_scale", None) is not None and args.class_id is None:
         p.error("--cfg_scale needs --class_id: guidance contrasts the class labels with the null label")
@@ -287,6 +317,15 @@ def get_args(argv=None):
             p.error("--unipc_steps needs --parametrization predict_noise or predict_original")
         if args.unipc_steps < 2:
             p.error("--unipc_steps needs at least 2 grid points (one model evaluation)")
+    if getattr(args, "sde_dpm_solver_steps", None) is not None:
+        if args.use_ddim or getattr(args, "dpm_solver_steps", None) is not None or \
+                getattr(args, "unipc_steps", None) is not None:
+            p.error("--sde_dpm_solver_steps, --use_ddim, --dpm_solver_steps and --unipc_steps select different "
+                    "samplers: give one of them")
+        if args.parametrization == "predict_previous":
+            p.error("--sde_dpm_solver_steps needs --parametrization predict_noise or predict_original")
+        if args.sde_dpm_solver_steps < 2:
+            p.error("--sde_dpm_solver_steps needs at least 2 grid points (one model evaluation)")
     return args
 
 
@@ -342,6 +381,8 @@ def main(argv=None):
             extra["dpm_solver_steps"] = args.dpm_solver_steps
         if getattr(args, "unipc_steps", None) is not None:
             extra["unipc_steps"] = args.unipc_steps
+        if getattr(args, "sde_dpm_solver_steps", None) is not None:
+            extra["sde_dpm_solver_steps"] = args.sde_dpm_solver_steps
         if "autoencoder" in cfg and hi > lo:  # sampler.py:320-325
             autoencoder = get_autoencoder(cfg["autoencoder"]["autoencoder_checkpoint_path"])
         D.barrier()  # every rank has loaded its models: the clock starts together

@@ -105,8 +105,8 @@ int ddb_ee_forward(ddb_model* m, const float* x_dev, const float* t_dev, const i
  *   mode 1: (c1*out + c0*x) + sigma*z (predict_original / predict_previous),
  *   mode 2: (c0*(x - c1*out) + d*out) + sigma*z (DDIM, sampler.py:112-120; sigma holds the reference's sigma_t^2).
  *   z_dev: this step's noise [n] or NULL (Philox from `seed`); ignored at t == 0 (z = 0).
- *   Mode 3 (DPM-Solver++) needs the previous step's data prediction and fails with DDB_ERR_INVALID here; so does
- *   mode 4 (UniPC), which needs the previous two. */
+ *   Mode 3 (DPM-Solver++) needs the previous step's data prediction and fails with DDB_ERR_INVALID here; so do
+ *   mode 4 (UniPC), which needs the previous two, and mode 5 (SDE-DPM-Solver++). */
 int ddb_ddpm_step(float* x_dev, const float* model_out_dev, const float* z_dev, const float* coef_dev, int32_t t,
                   int32_t mode, uint64_t seed, int64_t n, void* stream);
 
@@ -128,7 +128,13 @@ int ddb_ddpm_step(float* x_dev, const float* model_out_dev, const float* z_dev, 
  *     x' = px*xc + p0*D (predictor order 1), ... + p1*D1 (order 2);  then xb <- xc, D2 <- D1, D1 <- D.
  *   The sampler owns xb, D1 and D2 [B,C,H,W]; they persist across ddb_sampler_run_list calls like D_prev of mode 3
  *   (a row with corrector order 0 starts a new history).  Mode 4 runs only through ddb_sampler_run_list over
- *   timesteps whose row has predictor order 1 or 2, and is rejected with early exit. */
+ *   timesteps whose row has predictor order 1 or 2, and is rejected with early exit.
+ *   step_mode 5: SDE-DPM-Solver++(2M) (the reverse SDE, data prediction), coef_host [1000,8] with rows {a, b, rho,
+ *   phi, w0, w1, order, vs} (duodiff_b200.ddpm.sde_dpm_solver_coefficients): mode 3's update plus a noise term,
+ *     x' = (rho*x + phi*D) + vs*z  where vs != 0 (every step but the final one);  D_prev <- D_t.
+ *   z is the draw of the DDPM step at t: z_all_dev[t], or Philox keyed by (seed, t, global element index) as in
+ *   modes 0-2, so ddb_sampler_set_noise_offset shards it exactly.  D_prev, the order check, ddb_sampler_run_list only
+ *   and the rejection with early exit are as for mode 3. */
 int ddb_sampler_create(ddb_model* early, ddb_model* late, int32_t switch_t, int32_t B, const float* coef_host,
                        int32_t step_mode, float ee_threshold, int32_t ee_mode, ddb_sampler** out);
 void ddb_sampler_destroy(ddb_sampler* s);
@@ -157,16 +163,16 @@ int ddb_sampler_profile_step(ddb_sampler* s, float* x_dev, const int64_t* y_dev,
  *   the samples STILL IN THE BATCH at that layer (the reference's batch mean needs the dead layers evaluated).
  *   use_graph != 0 replays one captured CUDA graph per backbone (eps/x traces must then be NULL).  The captured step
  *   only touches sampler-owned memory (x, labels and logs are staged), so caller pointers may change between calls.
- *   Fails with DDB_ERR_INVALID for a step_mode 3 or 4 sampler (DPM-Solver++ and UniPC are defined over their grid
- *   only). */
+ *   Fails with DDB_ERR_INVALID for a step_mode 3, 4 or 5 sampler (DPM-Solver++, UniPC and SDE-DPM-Solver++ are
+ *   defined over their grid only). */
 int ddb_sampler_run(ddb_sampler* s, float* x_dev, const int64_t* y_dev, const float* z_all_dev, uint64_t seed,
                     int32_t t_first, int32_t t_last, float* eps_trace_dev, float* x_trace_dev,
                     int32_t* exit_idx_trace_dev, float* score_mean_trace_dev, int32_t use_graph, void* stream);
 /* Same loop over an explicit list of timesteps (host arrays of n_steps entries): the model runs at t_list[k] on the
  * late backbone when late[k] != 0, then the sampler's update rule is applied with the coefficients of t_list[k].
  * Used for the DDIM branch (sampler.py:103-126: strided schedule, hand-off `t < 1000 - t_switch` after the step) and
- * for DPM-Solver++ (step_mode 3) and UniPC (step_mode 4) over the same grid: a timestep whose table row has
- * (predictor) order 0 fails with DDB_ERR_INVALID (so does ddb_sampler_profile_step). */
+ * for DPM-Solver++ (step_mode 3), UniPC (step_mode 4) and SDE-DPM-Solver++ (step_mode 5) over the same grid: a
+ * timestep whose table row has (predictor) order 0 fails with DDB_ERR_INVALID (so does ddb_sampler_profile_step). */
 int ddb_sampler_run_list(ddb_sampler* s, float* x_dev, const int64_t* y_dev, const float* z_all_dev, uint64_t seed,
                          const int32_t* t_list_host, const uint8_t* late_host, int32_t n_steps, float* eps_trace_dev,
                          float* x_trace_dev, int32_t use_graph, void* stream);
